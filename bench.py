@@ -2,7 +2,7 @@
 """Benchmark of the SAT decoder hot path on B200 (BASELINE.json metric: captions/sec for the train step and greedy / beam
 decode at 1/2/4/8 GPUs, step p50 ms).
 
-    python bench.py --gpus N --steps K --warmup W [--workload all|train|c3|greedy|beam] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload all|train|c3|greedy|beam] [--impl reference] [--dump-outputs DIR]
 
 The line's headline (`value`, `e2e`, `roofline`, `cpu_baseline`) is BASELINE.json configs[1]: SAT resnet50 encoder, L=196,
 D=512, hidden 512, vocab 6400, batch 256 per GPU, bf16 training step (encoder fwd + decoder fwd + loss + full backward +
@@ -17,6 +17,16 @@ decode shards by image with no collective.  Times are CUDA-event times, max over
 `--impl reference` times the UNMODIFIED reference (model.py / util.py, copied into the git-ignored oracle/_ref/ by
 __graft_entry__.build(); the oracle port when that copy is absent) on the host CPU on a bounded sample of each workload.
 Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` (B200 arm, rank 0) writes what each workload's timed step computed in its last timed step to
+DIR/<workload>.<output>.npy, float32 or float64, so that two builds run with the same arguments (hence the same seeded inputs)
+can be compared output for output:
+  train / c3     loss, aux (the 8 step statistics of fused_loss), grad.<parameter> for every decoder parameter and
+                 grad.encoder (all encoder gradients, flattened and concatenated)
+  greedy / beam  tokens [B, S+1] (-1 past the caption's end), lengths, scores, perplexities and alphas [B, S+1, L] (0 past the
+                 end) of the returned caption of every image, as SAT.caption returns them
+An output of more than DUMP_SAMPLE elements is stored as the DUMP_SAMPLE elements at fixed flat indices (drawn from a generator
+seeded with 0, sorted); all files together stay under 64 MB.
 """
 import argparse
 import json
@@ -45,6 +55,8 @@ CFG = {
 }
 # bounded CPU samples of the same workloads (captions per timed step of the reference arm / cpu_baseline)
 CPU_SAMPLE = {"train": 16, "c3": 8, "greedy": 8, "beam": 4}
+DUMP_SAMPLE = 1 << 18
+DUMP_MAX_BYTES = 64 << 20
 
 
 def vocab(V):
@@ -171,7 +183,7 @@ def load_traffic(workload):
 
 
 # ------------------------------------------------------------------------------------------------
-# reference arm / cpu baseline: the unmodified reference (oracle/_ref or /root/reference) on the host cores
+# reference arm / cpu baseline: the unmodified reference (SAT_REFERENCE_DIR or oracle/_ref) on the host cores
 # ------------------------------------------------------------------------------------------------
 def _reference_model(c):
     """(kind, SAT module) -- kind 'reference' = the unmodified reference's SAT driven through oracle/ref_harness, with the
@@ -366,6 +378,60 @@ def timed(D, fn, steps, warmup, drain=None):
     return D.max_ms(evs[0].elapsed_time(evs[steps])), per
 
 
+def dump_array(x):
+    """host float32 / float64 copy of an output; above DUMP_SAMPLE elements, the fixed seeded sample of its flattened elements"""
+    x = x.detach()
+    if x.numel() > DUMP_SAMPLE:
+        idx = torch.randint(0, x.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        x = x.reshape(-1)[idx.to(x.device)]
+    x = x.cpu()
+    return (x if x.dtype == torch.float64 else x.float()).numpy()
+
+
+def train_outputs(model, loss, aux):
+    """what the last timed train step computed: its loss and statistics, and the parameter gradients it left"""
+    out = {"loss": dump_array(loss), "aux": dump_array(aux)}
+    enc = []
+    for n, p in model.named_parameters():
+        if p.grad is None:
+            continue
+        if n.startswith("encoder."):
+            enc.append(p.grad.reshape(-1).float())
+        else:
+            out["grad." + n] = dump_array(p.grad)
+    if enc:
+        out["grad.encoder"] = dump_array(torch.cat(enc))
+    return out
+
+
+def decode_outputs(t, c):
+    """the returned caption of every image of the last timed decode (decode.assemble, as SAT.caption returns them), padded to
+    arrays"""
+    import numpy as np
+    from sat_b200 import decode
+    caps, scores, alphas, ppls = decode.assemble(t, (c["size"], c["size"]))
+    B, W = len(caps), c["S"] + 1
+    tokens = torch.full((B, W), -1.0)
+    alpha = torch.zeros(B, W, c["L"])
+    for i, (cap, a) in enumerate(zip(caps, alphas)):
+        tokens[i, :len(cap)] = torch.tensor(cap, dtype=torch.float32)
+        alpha[i, :a.shape[0]] = a.reshape(a.shape[0], c["L"])
+    return {"tokens": dump_array(tokens), "lengths": np.array([len(x) for x in caps], dtype=np.float32),
+            "scores": np.array(scores, dtype=np.float64), "perplexities": np.array(ppls, dtype=np.float64),
+            "alphas": dump_array(alpha)}
+
+
+def write_outputs(path, outputs):
+    import numpy as np
+    arrays = {"%s.%s" % (w, k): v for w, o in outputs.items() for k, v in o.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_MAX_BYTES))
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v)
+
+
 def roof_entry(kernel, bound, work, ms, n, peak, unit, traffic, traffic_keys=None, **extra):
     """`traffic`: the committed ncu capture of THIS workload ({} = none: traffic null); traffic_keys: entries of it to sum
     (default: the kernel's own name)"""
@@ -385,7 +451,7 @@ def roof_entry(kernel, bound, work, ms, n, peak, unit, traffic, traffic_keys=Non
     return e
 
 
-def run_train(args, D, name):
+def run_train(args, D, name, outputs=None):
     from sat_b200 import _lib, decoder
     from sat_b200.dist import OverlappedGradReducer
     from sat_b200.model import SAT
@@ -420,9 +486,12 @@ def run_train(args, D, name):
             reducer.finish()
         opt.step()
 
+    last = {}
+
     def step_device():
         loss, aux = model.fused_loss((img_d.clone(), caps_d, lens_d))
         backward_and_step(loss)
+        last["loss"], last["aux"] = loss, aux
         return loss
 
     # End-to-end step = what a training loop around the public API does: the NEXT batch's host->device copy is issued on a
@@ -472,6 +541,8 @@ def run_train(args, D, name):
     clocks.start()
     tot_ms, per = timed(D, step_device, args.steps, args.warmup)
     clk = clocks.stop()
+    if outputs is not None:
+        outputs[name] = train_outputs(model, last["loss"], last["aux"])
     launches = (_lib.launch_count() - l0) * args.steps // (args.steps + args.warmup)
     value = B * world * args.steps / (tot_ms * 1e-3)
     e2e_ms, _ = timed(D, step_e2e, args.steps, args.warmup, drain=drain_e2e)
@@ -561,7 +632,7 @@ def run_train(args, D, name):
     return rec
 
 
-def run_decode(args, D, name):
+def run_decode(args, D, name, outputs=None):
     from sat_b200 import _lib, decode, decoder
     from sat_b200.model import SAT
     c = CFG[name]
@@ -579,8 +650,11 @@ def run_decode(args, D, name):
     bld = decoder.annotations_as_bld(ann, dw.pw.dtype)
     voc = dict(PAD=0, UNK=c["V"] - 3, START=c["V"] - 2, END=c["V"] - 1)
 
+    last = {}
+
     def step_device():
-        return decode.decode_annotations(dw, bld, c["k"], c["S"], 1.0, None, 0.5, voc)
+        last["t"] = decode.decode_annotations(dw, bld, c["k"], c["S"], 1.0, None, 0.5, voc)
+        return last["t"]
 
     def step_e2e():
         # public bulk-captioning call: pinned host images in chunks of 256 (encoder activation memory); copies, kernels
@@ -593,11 +667,12 @@ def run_decode(args, D, name):
     clocks.start()
     tot_ms, per = timed(D, step_device, args.steps, args.warmup)
     clk = clocks.stop()
+    if outputs is not None:
+        outputs[name] = decode_outputs(last["t"], c)
     launches = (_lib.launch_count() - l0) * args.steps // (args.steps + args.warmup)
     value = B * world * args.steps / (tot_ms * 1e-3)
-    e2e_steps = max(2, args.steps // 3)
-    e2e_ms, _ = timed(D, step_e2e, e2e_steps, 1)
-    e2e_value = B * world * e2e_steps / (e2e_ms * 1e-3)
+    e2e_ms, _ = timed(D, step_e2e, args.steps, 1)
+    e2e_value = B * world * args.steps / (e2e_ms * 1e-3)
 
     _lib.profile_begin(1)
     for _ in range(2):
@@ -623,8 +698,8 @@ def run_decode(args, D, name):
         "step_p50_ms": statistics.median(per), "dtype": "bf16" if args.precision == "bf16" else "f32",
         "config": config_dict(name, c, B, world), "clocks": clk,
         "e2e": {"value": e2e_value, "unit": "captions/s", "h2d_bytes_per_step": img_h.numel() * 4,
-                "d2h_bytes_per_step": int(B * (c["S"] + 1) * 4 * 2 + B * c["S"] * c["L"] * 4), "ms_per_step": e2e_ms / e2e_steps,
-                "steps": e2e_steps},
+                "d2h_bytes_per_step": int(B * (c["S"] + 1) * 4 * 2 + B * c["S"] * c["L"] * 4), "ms_per_step": e2e_ms / args.steps,
+                "steps": args.steps},
         "gpu_launches": int(launches), "roofline": roof,
     }
     del model, dw, bld, ann
@@ -636,8 +711,11 @@ def run_b200(args):
     D = Dist()
     names = ["train", "c3", "greedy", "beam"] if args.workload == "all" else [args.workload]
     recs = {}
+    outputs = {} if (args.dump_outputs and D.rank == 0) else None
     for n in names:
-        recs[n] = run_train(args, D, n) if CFG[n]["kind"] == "train" else run_decode(args, D, n)
+        recs[n] = run_train(args, D, n, outputs) if CFG[n]["kind"] == "train" else run_decode(args, D, n, outputs)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     head = names[0]
     line = {"metric": METRIC, "n_gpus": D.world, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "data": "synthetic"}
     line.update(recs[head])
@@ -669,7 +747,13 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch of the train workload (default: the BASELINE config's)")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each workload's last timed step computed to DIR/<workload>.<output>.npy (B200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 arm")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

@@ -1,6 +1,6 @@
-"""Generate tests/golden/*.npz from the UNMODIFIED reference (run by hand in the build container:
-`python oracle/make_golden.py`).  Test infrastructure only; needs /root/reference, which does not
-exist on the GPU box -- the committed .npz files are what travels.
+"""Generate tests/golden/*.npz from the UNMODIFIED reference (run by hand: `python oracle/make_golden.py [c1|layers|api]`).
+Test infrastructure only; needs the upstream model.py / util.py (SAT_REFERENCE_DIR or oracle/_ref/, see ref_harness.py), which
+the repository does not contain -- the committed .npz files are what the tests read.
 
 Every case drives the reference's own public methods (SAT.train_batch, SAT.criterion, the
 doubly-stochastic term exactly as training_step writes it, SAT.caption) with the CNN trunk replaced
@@ -20,6 +20,18 @@ from oracle import ref_harness as rh  # noqa: E402
 
 warnings.filterwarnings("ignore")
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# cases larger than 1 MB in one file: the arrays under the prefix go to <name>.<part>.npz (tests/conftest.py:golden_arrays
+# reads both)
+SPLIT = {"train_layers3": ("grads", "G/"), "c1_resnet18": ("decode", "decode/")}
+
+
+def save(name, out):
+    part, prefix = SPLIT.get(name, (None, None))
+    if part is None:
+        np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+        return
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **{k: v for k, v in out.items() if not k.startswith(prefix)})
+    np.savez_compressed(os.path.join(OUT, "%s.%s.npz" % (name, part)), **{k: v for k, v in out.items() if k.startswith(prefix)})
 
 
 def build(model, seed, D, A, E, H, V, label_smoothing=0.0, att_gamma=1.0, sharpen=None, layers=1):
@@ -79,7 +91,7 @@ def train_case(model, name, seed, B_img, ncap, hw, D, A, E, H, V, T, ragged, lab
                     loss=np.float64(loss.item()), ce=np.float64(ce.item()), acc=np.float64(acc.item()),
                     d_ann=ann.grad.numpy().copy(), label_smoothing=np.float64(label_smoothing),
                     att_gamma=np.float64(1.0), dims=np.array([D, A, E, H, V, T, hw[0], hw[1], ncap])))
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+    save(name, out)
     print(name, "loss", loss.item(), "acc", acc.item(), "tokens", lp.data.shape[0])
 
 
@@ -113,7 +125,7 @@ def decode_case(model, name, seed, n_img, hw, D, A, E, H, V, max_len, sharpen, l
     for i in range(n_img):
         out["k3_LN_T0.7/n%d/tokens" % i] = np.array(caps[i], dtype=np.int64)
         out["k3_LN_T0.7/n%d/score" % i] = np.float64(scores[i])
-    np.savez_compressed(os.path.join(OUT, name + ".npz"), **out)
+    save(name, out)
     print(name, {k: v for k, v in lens.items() if k.endswith("None_best") or k.endswith("LN_best")})
 
 
@@ -219,8 +231,71 @@ def c1_case(model):
             out["decode/k%d/n%d/score" % (k, i)] = np.float64(scores[i])
             out["decode/k%d/n%d/alpha_sum" % (k, i)] = alph[i].sum(0).numpy()
         print("c1 decode k=%d lengths" % k, [len(c) for c in caps_o])
-    np.savez_compressed(os.path.join(OUT, "c1_resnet18.npz"), **out)
+    save("c1_resnet18", out)
     print("c1_resnet18 loss", loss.item(), "training_step loss", float(ts["loss"]), "acc", acc.item())
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# the module surface around the decoder (tests/test_model_api.py, tests/test_callers_cpu.py use the same hparams and inputs):
+#   * init/:  state_dict keys, shapes and per-tensor digests (norm + 64 sampled entries) of SAT(**default_hparams(vocab_size=400))
+#             under torch.manual_seed(3);
+#   * score/: score_captions' cosine similarity and result keys;
+#   * lr/:    learning rates of every param group over 3 epochs x 6 batches of warm-up + scheduler stepping, per scheduler.
+# The committed reference_api.npz was recorded by running api_case on sat_b200.model (it takes any module with the reference's
+# SAT API), at a commit whose `reference`-marked tests passed against the upstream files: state_dict bit-identical, learning
+# rates within 1e-12, cosine similarity within 1e-6.  With the upstream files present, `python oracle/make_golden.py api`
+# records it from the reference itself.
+# ------------------------------------------------------------------------------------------------------------------
+def reference_lrs(model, sched):
+    """the reference's optimizer / scheduler driven like its training loop: training_step's warm-up and per-batch stepping
+    (model.py:608-617), the epoch hooks (model.py:633-635) -> (initial lrs, [steps, groups] lrs, scheduler class name)"""
+    ref = model.SAT(**dict(rh.small_hparams(scheduler=sched, **rh.LR_EXTRA)))
+    ro = ref.configure_optimizers()
+    ref._optimizer = ro
+    init = [pg["lr"] for pg in ro.param_groups]
+    tr = type("T", (), {"global_step": 0})()
+    ref.trainer = tr
+    lrs = []
+    for epoch in range(3):
+        for it in range(6):
+            if tr.global_step < ref.hparams.lr_warmup_steps:
+                lr_scale = min(1, float(tr.global_step + 1) / ref.hparams.lr_warmup_steps)
+                for pg, init_lr in zip(ro.param_groups, ref.opt_init_lr):
+                    pg["lr"] = lr_scale * init_lr
+            elif tr.global_step > 0 and type(ref.scheduler) in (torch.optim.lr_scheduler.CosineAnnealingWarmRestarts, torch.optim.lr_scheduler.OneCycleLR):
+                ref.scheduler.step()
+            ro.step()
+            lrs.append([pg["lr"] for pg in ro.param_groups])
+            tr.global_step += 1
+        ref.current_epoch = epoch
+        ref.training_epoch_end([{"loss": 1.0}])
+        if sched == "plateau":
+            ref.hparams.plateau_monitor = ref.hparams.save_monitor = ref.hparams.early_stop_monitor = "bleu4"
+            ref.validation_epoch_end([{"bleu4": 0.1}])
+    return init, lrs, type(ref.scheduler).__name__
+
+
+def api_case(model):
+    out = {}
+    torch.manual_seed(3)
+    sd = model.SAT(**rh.default_hparams(vocab_size=400)).state_dict()
+    out["init/keys"] = np.array(list(sd.keys()))
+    for k, v in sd.items():
+        flat = v.reshape(-1)
+        out["init/shape/" + k] = np.array(v.shape, dtype=np.int64)
+        out["init/norm/" + k] = np.float64(flat.double().norm().item())
+        out["init/samp/" + k] = flat[digest_indices(flat.numel())].numpy().copy()
+    torch.manual_seed(3)
+    r = model.SAT(**rh.small_hparams()).score_captions(*rh.score_inputs())
+    out["score/cosine_similarity"] = np.float64(r["cosine_similarity"])
+    out["score/keys"] = np.array(sorted(r.keys()))
+    for sched in rh.LR_SCHEDULERS:
+        init, lrs, name = reference_lrs(model, sched)
+        out["lr/%s/init" % sched] = np.array(init, dtype=np.float64)
+        out["lr/%s/lrs" % sched] = np.array(lrs, dtype=np.float64)
+        out["lr/%s/scheduler" % sched] = np.array(name)
+    save("reference_api", out)
+    print("reference_api", len(sd), "state_dict entries, cosine", out["score/cosine_similarity"])
 
 
 def layers_cases(model):
@@ -242,6 +317,8 @@ def main():
         return c1_case(model)
     if len(sys.argv) > 1 and sys.argv[1] == "layers":
         return layers_cases(model)
+    if len(sys.argv) > 1 and sys.argv[1] == "api":
+        return api_case(model)
     # tiny, ragged, 2 captions per image, non-square map, label smoothing, peaky attention
     train_case(model, "train_tiny", 0, B_img=3, ncap=2, hw=(3, 4), D=16, A=8, E=10, H=14, V=50, T=6,
                ragged=True, label_smoothing=0.1, sharpen=dict(fatt=20.0))
@@ -258,6 +335,7 @@ def main():
                 sharpen=dict(wo=8.0, emb=2.0, fatt=30.0, end_bias=3.0))
     layers_cases(model)
     c1_case(model)
+    api_case(model)
 
 
 if __name__ == "__main__":

@@ -1,12 +1,11 @@
-"""Test infrastructure only: load the UNMODIFIED reference (/root/reference/model.py)
-in this container so golden vectors can be generated from it.
+"""Test infrastructure only: load the UNMODIFIED reference (the upstream model.py / util.py, from
+SAT_REFERENCE_DIR or oracle/_ref/) so golden vectors can be generated from it.
 
 The reference imports `pytorch_lightning` and `nltk` at module import time
 (model.py:1-4, util.py:7-8); neither is installed in this image, so tiny stand-in
 modules are injected into sys.modules first.  Nothing here is used by the product
-path, and `/root/reference` does not exist on the GPU box, so only
-`oracle/make_golden.py` (run by hand in the build container) and the
-`reference`-marked CPU tests import this file.
+path; `oracle/make_golden.py` (run by hand), bench.py's reference arm and the CPU tests import
+this file (the tests for its shared inputs; only the `reference`-marked ones load the reference).
 """
 import inspect
 import os
@@ -17,11 +16,11 @@ import torch
 from torch import nn
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# /root/reference exists in the build container only.  __graft_entry__.build() copies the reference's model.py / util.py
-# UNMODIFIED into the git-ignored oracle/_ref/ (it travels to the GPU box like the built .so), so that bench.py's
-# `--impl reference` arm can time the real reference there.  Nothing under oracle/_ref is ever committed.
-_CANDIDATES = [os.environ.get("SAT_REFERENCE_DIR", ""), "/root/reference", os.path.join(_HERE, "_ref")]
-REFERENCE_DIR = next((d for d in _CANDIDATES if d and os.path.isfile(os.path.join(d, "model.py"))), "/root/reference")
+# The repository does not contain the reference.  SAT_REFERENCE_DIR names a checkout of it; __graft_entry__.build() copies
+# that checkout's model.py / util.py UNMODIFIED into the git-ignored oracle/_ref/, which travels with the built tree, so that
+# bench.py's `--impl reference` arm can time the real reference there.  Nothing under oracle/_ref is ever committed.
+_CANDIDATES = [os.environ.get("SAT_REFERENCE_DIR", ""), os.path.join(_HERE, "_ref")]
+REFERENCE_DIR = next((d for d in _CANDIDATES if d and os.path.isfile(os.path.join(d, "model.py"))), os.path.join(_HERE, "_ref"))
 
 
 class _HParams(dict):
@@ -163,3 +162,27 @@ def default_hparams(**over):
     hp.setdefault("vocab_stoi", stoi)
     hp.setdefault("vocab_itos", itos)
     return hp
+
+
+# inputs shared by oracle/make_golden.py api_case and the tests that read its golden file (tests/test_callers_cpu.py)
+LR_SCHEDULERS = ["step", "exp", "cosine", "one_cycle", "plateau"]
+LR_EXTRA = dict(epochs=3, train_loader_len=6, lr_warmup_steps=4, cosine_iterations=5, cosine_multi=2, min_lr=1e-6, accumulate=1,
+                milestones=[1, 2], lr_gamma=0.5, plateau_patience=0, one_cycle_pct=0.3, one_cycle_div=10.0, one_cycle_fdiv=100.0,
+                encoder_finetune_after=1, momentum=0.9, nesterov=False)
+
+
+def small_hparams(**over):
+    hp = default_hparams(encoder_arch="resnet18", encoder_dim=64, attention_dim=32, embed_dim=32, decoder_dim=64, vocab_size=128,
+                         input_size=64)
+    hp.update(over)
+    return hp
+
+
+def score_inputs():
+    """(captions, encoded captions, lengths, perplexities) arguments of SAT.score_captions"""
+    g = torch.Generator().manual_seed(4)
+    enc = torch.randint(1, 124, (5, 3, 9), generator=g)
+    enc[:, :, 0] = 126
+    lens = torch.randint(2, 8, (5, 3), generator=g)
+    caps = [torch.randint(1, 124, (int(n),), generator=g).tolist() for n in (3, 7, 1, 5, 4)]
+    return caps, enc, lens, [1.0, 2.0, 3.0, 4.0, 5.0]

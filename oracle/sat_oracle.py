@@ -8,7 +8,7 @@ and has no CPU fallback.
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4), so the
 oracle is pinned against OUTPUTS OF THE REFERENCE ITSELF, generated in the build container
-by `oracle/make_golden.py` (imports the unmodified /root/reference/model.py through
+by `oracle/make_golden.py` (imports the unmodified upstream model.py through
 `oracle/ref_harness.py`) and committed under `tests/golden/`.  `tests/test_oracle_golden.py`
 checks every function here against those vectors (forward, loss, gradients via autograd,
 greedy and beam token ids, scores, alphas, perplexities).

@@ -1,5 +1,5 @@
 """GPU parity at BASELINE configs[0] (C1: resnet18 trunk + readme resize -> L=196, D=512, A=128, E=256, H=512, V=6400, batch 8,
-20 targets, fp32) against outputs of the UNMODIFIED reference (tests/golden/c1_resnet18.npz, oracle/make_golden.py::c1_case).
+20 targets, fp32) against outputs of the UNMODIFIED reference (tests/golden/c1_resnet18*.npz, oracle/make_golden.py::c1_case).
 The fixture stores seeds instead of weights / images: the module's seeded default init is bit-identical to the reference's
 (tests/test_model_api.py) and the inputs come from seeded CPU generators.
 
@@ -7,15 +7,13 @@ The fixture stores seeds instead of weights / images: the module's seeded defaul
   gradients (digests) <= 2e-5, greedy and beam-5 token ids bit-exact incl. early <END> and shrinking beams;
 * the whole SAT.training_step with the real trunk on cuDNN (TF32 off): loss within 1e-4 of the reference's CPU step
   (convolution rounding differs between cuDNN and the CPU's oneDNN; the decoder itself is checked at 1e-5 above)."""
-import os
 import warnings
 
-import numpy as np
 import pytest
 import torch
 from torch import nn
 
-from conftest import GOLDEN
+from conftest import golden_arrays
 from oracle import ref_harness as rh
 from test_train_forward_gpu import relerr
 
@@ -60,7 +58,7 @@ def model(seed=0, sharpen=False):
 
 @pytest.fixture(scope="module")
 def gold():
-    return np.load(os.path.join(GOLDEN, "c1_resnet18.npz"))
+    return golden_arrays("c1_resnet18")
 
 
 def test_c1_decoder_forward_backward_on_reference_annotations(gold):

@@ -67,6 +67,21 @@ def test_score_captions_cosine_similarity_matches_reference():
     assert 0 <= b["bleu4"] <= b["bleu1"] <= 1 and 0 <= b["gleu"] <= 1
 
 
+def test_score_captions_cosine_similarity_matches_reference_golden():
+    """the same check against the reference's result in tests/golden/reference_api.npz (oracle/make_golden.py api)"""
+    import sat_b200  # noqa: F401
+    from conftest import golden_arrays
+    from sat_b200.model import SAT
+    z = golden_arrays("reference_api")
+    torch.manual_seed(3)
+    m = SAT(**small_hparams())
+    b = m.score_captions(*rh.score_inputs())
+    assert abs(float(z["score/cosine_similarity"]) - b["cosine_similarity"]) < 1e-6
+    assert sorted(b.keys()) == z["score/keys"].tolist()
+    assert b["perplexity"] == 3.0
+    assert 0 <= b["bleu4"] <= b["bleu1"] <= 1 and 0 <= b["gleu"] <= 1
+
+
 @pytest.mark.reference
 @pytest.mark.parametrize("sched", ["step", "exp", "cosine", "one_cycle", "plateau"])
 def test_lr_schedule_and_warmup_match_reference(sched):
@@ -111,6 +126,35 @@ def test_lr_schedule_and_warmup_match_reference(sched):
             ref.validation_epoch_end([{"bleu4": 0.1}])
             mine.validation_epoch_end([{"bleu4": 0.1}])
     assert np.allclose(np.array(lrs_r), np.array(lrs_m), rtol=1e-12, atol=0)
+
+
+@pytest.mark.parametrize("sched", ["step", "exp", "cosine", "one_cycle", "plateau"])
+def test_lr_schedule_and_warmup_match_reference_golden(sched):
+    """the same learning-rate trajectory check against the reference's rates in tests/golden/reference_api.npz
+    (oracle/make_golden.py api: the reference's optimizer and scheduler driven like its training loop)"""
+    import sat_b200  # noqa: F401
+    from conftest import golden_arrays
+    from sat_b200.model import SAT
+    z = golden_arrays("reference_api")
+    mine = SAT(**dict(small_hparams(scheduler=sched, **rh.LR_EXTRA)))
+    mo = mine.configure_optimizers()
+    assert type(mine.scheduler).__name__ == str(z["lr/%s/scheduler" % sched])
+    assert [pg["lr"] for pg in mo.param_groups] == z["lr/%s/init" % sched].tolist()
+    tr = type("T", (), {"global_step": 0})()
+    mine.trainer = tr
+    lrs_m = []
+    for epoch in range(3):
+        for it in range(6):
+            mine._step_lr_schedule()
+            mo.step()
+            lrs_m.append([pg["lr"] for pg in mo.param_groups])
+            tr.global_step += 1
+        mine.current_epoch = epoch
+        mine.training_epoch_end([{"loss": 1.0}])
+        if sched == "plateau":
+            mine.hparams.plateau_monitor = mine.hparams.save_monitor = mine.hparams.early_stop_monitor = "bleu4"
+            mine.validation_epoch_end([{"bleu4": 0.1}])
+    assert np.allclose(np.array(lrs_m), z["lr/%s/lrs" % sched], rtol=1e-12, atol=0)
 
 
 def test_load_from_checkpoint_pl_format(tmp_path):

@@ -1,5 +1,5 @@
 """CPU checks of the drop-in module surface (model.py:134-212): parameter names/shapes, seeded default
-init identical to the reference (needs /root/reference), vocabulary helpers."""
+init identical to the reference (against its golden digests; live when the upstream files are present), vocabulary helpers."""
 import warnings
 
 import pytest
@@ -27,6 +27,27 @@ def test_state_dict_and_seeded_init_match_reference():
     for k in sa:
         assert sa[k].shape == sb[k].shape and torch.equal(sa[k], sb[k]), k
     b.load_state_dict(sa)          # a reference checkpoint loads into the new module
+
+
+def test_state_dict_and_seeded_init_match_reference_golden():
+    """the same check against tests/golden/reference_api.npz (oracle/make_golden.py api): keys in order, shapes, and per-tensor
+    digests (norm + 64 sampled entries, exact) of the reference's seeded init"""
+    from conftest import golden_arrays
+    from sat_b200.model import SAT
+    z = golden_arrays("reference_api")
+    torch.manual_seed(3)
+    sb = SAT(**small_hp()).state_dict()
+    keys = z["init/keys"].tolist()
+    assert list(sb.keys()) == keys
+    for k in keys:
+        flat = sb[k].reshape(-1)
+        assert tuple(sb[k].shape) == tuple(z["init/shape/" + k].tolist()), k
+        idx = torch.randint(0, flat.numel(), (64,), generator=torch.Generator().manual_seed(7 + flat.numel() % 1000))
+        assert torch.equal(flat[idx], torch.from_numpy(z["init/samp/" + k])), k
+        ref_norm = float(z["init/norm/" + k])
+        assert abs(float(flat.double().norm()) - ref_norm) <= 1e-12 * ref_norm, k
+    # a checkpoint with the reference's keys and shapes loads into the new module
+    SAT(**small_hp()).load_state_dict({k: torch.zeros(tuple(z["init/shape/" + k].tolist()), dtype=sb[k].dtype) for k in keys})
 
 
 def test_surface_and_helpers():

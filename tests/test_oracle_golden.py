@@ -1,5 +1,5 @@
 """Pins oracle/sat_oracle.py against outputs of the unmodified reference (tests/golden/*.npz,
-made by oracle/make_golden.py from /root/reference/model.py).  CPU only."""
+made by oracle/make_golden.py from the upstream model.py).  CPU only."""
 import numpy as np
 import pytest
 import torch
