@@ -1,7 +1,8 @@
 """CPU oracle for the Show-Attend-and-Tell decoder hot path.
 
 TEST INFRASTRUCTURE ONLY.  This is a plain-torch (CPU, fp32 or fp64) restatement of the
-algorithm in the reference's model.py / util.py.  Only `tests/`, `__graft_entry__.smoke()`
+algorithm in the reference's model.py / util.py.  `train_batch` / `train_loss` also run on a CUDA device when the inputs
+live there (the full-batch float64 references of tests/test_full_size_grads_gpu.py).  Only `tests/`, `__graft_entry__.smoke()`
 and `bench.py`'s cpu_baseline / `--impl reference` legs may import it, and only as the
 checker or as the timed CPU baseline.  The product path (`sat_b200`) never imports this file
 and has no CPU fallback.
@@ -157,9 +158,9 @@ def train_batch(W, ann_img, encoded_captions, lengths, epsilon=1.0, deep=True, r
     else:
         h, c = init_lstm(W, ann)
     h, c = h.clone(), c.clone()
-    dt = ann.dtype
-    logits = torch.zeros(B, T, V, dtype=dt)
-    alphas = torch.zeros(B, T, L, dtype=dt)
+    dt, dev = ann.dtype, ann.device
+    logits = torch.zeros(B, T, V, dtype=dt, device=dev)
+    alphas = torch.zeros(B, T, L, dtype=dt, device=dev)
     for step in range(T):
         act = lens > step
         if not bool(act.any()):
@@ -178,8 +179,8 @@ def train_batch(W, ann_img, encoded_captions, lengths, epsilon=1.0, deep=True, r
         stacked = h.dim() == 3
         logit, alpha, h2, c2 = decoder_step(W, ann[idx], words, h[:, idx] if stacked else h[idx], c[:, idx] if stacked else c[idx],
                                             deep, ed, od)
-        alphas = alphas.index_put((idx, torch.tensor(step)), alpha)
-        logits = logits.index_put((idx, torch.tensor(step)), logit)
+        alphas = alphas.index_put((idx, torch.tensor(step, device=dev)), alpha)
+        logits = logits.index_put((idx, torch.tensor(step, device=dev)), logit)
         if stacked:
             h = h.index_copy(1, idx, h2)
             c = c.index_copy(1, idx, c2)
