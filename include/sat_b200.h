@@ -38,7 +38,7 @@ extern "C" {
 #define SAT_BF16 1
 #define SAT_ERR_INVALID (-1)
 
-#define SAT_ABI_VERSION 3
+#define SAT_ABI_VERSION 4
 #define SAT_MAX_LAYERS 4      /* decoder_layers (nn.LSTM num_layers, model.py:175-180) supported by the kernels */
 
 typedef struct SatDims {
@@ -214,10 +214,10 @@ typedef struct SatDecodeBuffers {
   void* z;               /* [R,D] s                                                               */
   void* gz;              /* [R,D] s                                                               */
   void* xo;              /* [R,E] s                                                               */
-  float* logits;         /* [R,V]                                                                 */
+  float* logits;         /* [R,V]  SAT_VOCAB_PATH_ROWS only, else NULL                           */
   float* alpha_all;      /* [S+1,R,L]  alpha of every step and row (histories hold row indices)    */
-  float* topk_stats;     /* [R, ceil(V/128), 4] or NULL: greedy (k = 1) tensor-core decode keeps per-tile soft-max statistics
-                                         and the best word instead of writing the logits                       */
+  float* topk_stats;     /* [R, ceil(V/128), 4] or NULL: the fused paths (sat_decode_vocab_path) keep per-tile soft-max statistics
+                                         (greedy: and the best word) instead of writing the logits             */
   float* cand_val;       /* [R,kcap]   per-row candidates: score (log-prob + parent score)        */
   int32_t* cand_idx;     /* [R,kcap]   word                                                       */
   float* cand_key;       /* [R,kcap]   sampling key (multinomial sampler), NULL for beam search   */
@@ -253,6 +253,13 @@ typedef struct SatDecodeBuffers {
   uint64_t sample_seed;  /* the sampling / noise draws are a pure function of (seed, step, row, word) */
   int32_t call_id;       /* non-zero tag of this call for done_host (distinguishes calls still in flight on the stream) */
   int32_t reserved1;
+  /* fused beam / sampling candidates (sat_decode_vocab_path() == SAT_VOCAB_PATH_CAND; NULL otherwise): the vocabulary GEMM's
+   * epilogue keeps per 128-column tile the soft-max statistics in topk_stats ([R, ceil(V/128), 4]: max and sum exp of x = logit / T)
+   * and the tile's best kcap candidate words, in (key descending, word ascending) order, instead of writing the logits */
+  float* tile_val;       /* [R, ceil(V/128), kcap]  x of the candidate; -inf in an empty slot                              */
+  int32_t* tile_idx;     /* [R, ceil(V/128), kcap]  word; 0x7fffffff in an empty slot                                       */
+  float* tile_key;       /* [R, ceil(V/128), kcap]  multinomial sampler: 20/step * x + Gumbel noise (the selection key), else NULL */
+  float* topk_stats2;    /* [R, ceil(V/128), 2]     multinomial sampler: max and sum exp of 20/step * x over the unmasked words */
 } SatDecodeBuffers;
 
 int sat_version(void);
@@ -369,6 +376,16 @@ int sat_train_param_grads(const SatDims* d, const SatTrainBuffers* b, const SatP
 
 /* GxV[v,:] = Emb[v,:] * Wihe^T + bg for every vocabulary entry (once per set of weights). */
 int sat_decode_prepare_weights(const SatDims* d, const SatWeights* w, float* GxV, void* stream);
+
+/* Which vocabulary stage sat_decode runs for these dims, beam width and sample method (0 beam, 1 multinomial, 2 topk), and so
+ * which buffers it reads: SAT_VOCAB_PATH_ROWS = [R,V] `logits` + the shared-memory row kernels (V <= 58,072; multinomial
+ * V <= 29,032), SAT_VOCAB_PATH_GREEDY = `topk_stats` (greedy on the bf16 tensor-core path), SAT_VOCAB_PATH_CAND = `topk_stats`
+ * + `tile_val` / `tile_idx` (+ `tile_key` / `topk_stats2` for the multinomial sampler): bf16 tensor-core decode where a logits
+ * row does not fit the row kernels, or everywhere under SAT_VOCAB_TOPK=1.  < 0 (error set) when no path takes the call. */
+#define SAT_VOCAB_PATH_ROWS 0
+#define SAT_VOCAB_PATH_GREEDY 1
+#define SAT_VOCAB_PATH_CAND 2
+int sat_decode_vocab_path(const SatDims* d, int32_t k, int32_t sample_method, int32_t sample_topk);
 
 /* Batched greedy (k = 1) / beam decode; d->B = n_img * k rows, d->Bi = n_img, d->ncap = k.  Runs
  * max_gen_length + 1 steps with device-side bookkeeping (no host sync); results are in the fin_* buffers. */

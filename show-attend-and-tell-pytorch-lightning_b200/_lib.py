@@ -55,7 +55,8 @@ class SatDecodeBuffers(C.Structure):
                [("k", C.c_int32), ("max_gen_length", C.c_int32), ("rescore", C.c_int32), ("reward", C.c_float),
                 ("tokPAD", C.c_int32), ("tokSTART", C.c_int32), ("tokEND", C.c_int32), ("tokUNK", C.c_int32),
                 ("sample_method", C.c_int32), ("sample_topk", C.c_int32), ("kcap", C.c_int32), ("decoder_noise", C.c_float),
-                ("sample_seed", C.c_uint64), ("call_id", C.c_int32), ("reserved1", C.c_int32)]
+                ("sample_seed", C.c_uint64), ("call_id", C.c_int32), ("reserved1", C.c_int32)] + \
+               [(n, vp) for n in ("tile_val", "tile_idx", "tile_key", "topk_stats2")]
 
 
 class SatParamGrads(C.Structure):
@@ -69,7 +70,8 @@ class SatParamGrads(C.Structure):
 EXPORTS = ["sat_version", "sat_last_error", "sat_abi_sizeof", "sat_launch_count", "sat_profile_begin", "sat_profile_end", "sat_dropout_multiplier", "sat_pack_weights",
            "sat_linear", "sat_linear_nt", "sat_prepare_images", "sat_resize_nhwc_fwd", "sat_resize_nhwc_bwd",
            "sat_attention_step_fwd", "sat_cast_captions", "sat_train_forward", "sat_train_backward", "sat_param_grads_workspace_bytes", "sat_train_param_grads",
-           "sat_decode_prepare_weights", "sat_decode"]
+           "sat_decode_prepare_weights", "sat_decode", "sat_decode_vocab_path"]
+VOCAB_PATH_ROWS, VOCAB_PATH_GREEDY, VOCAB_PATH_CAND = 0, 1, 2      # sat_decode_vocab_path
 
 _lib = None
 
@@ -125,6 +127,7 @@ def lib():
     L.sat_train_param_grads.argtypes = [C.POINTER(SatDims), C.POINTER(SatTrainBuffers), C.POINTER(SatParamGrads), vp, C.c_int64, vp]
     L.sat_decode_prepare_weights.argtypes = [C.POINTER(SatDims), C.POINTER(SatWeights), vp, vp]
     L.sat_decode.argtypes = [C.POINTER(SatDims), C.POINTER(SatWeights), C.POINTER(SatDecodeBuffers), vp]
+    L.sat_decode_vocab_path.argtypes = [C.POINTER(SatDims), C.c_int32, C.c_int32, C.c_int32]
     _lib = L
     return L
 

@@ -241,6 +241,13 @@ __host__ __device__ __forceinline__ float sat_dropout_scale(float p, uint64_t se
   const float u = (float)(sat_hash32(seed, stream, idx) >> 8) * (1.0f / 16777216.0f);
   return u < p ? 0.0f : 1.0f / (1.0f - p);
 }
+// sampling decoders: uniform in (0, 1) and standard Gumbel noise, pure functions of (seed, stream, idx)
+__device__ __forceinline__ float sat_uniform01(uint64_t seed, uint32_t stream, uint64_t idx) {
+  return ((float)(sat_hash32(seed, stream, idx) >> 8) + 0.5f) * (1.0f / 16777216.0f);
+}
+__device__ __forceinline__ float sat_gumbel(uint64_t seed, uint32_t stream, uint64_t idx) {
+  return -logf(-logf(sat_uniform01(seed, stream, idx)));
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -11,6 +11,27 @@
 
 namespace {
 
+constexpr size_t SMEM_LIMIT = 227 * 1024;
+size_t topk_smem_bytes(int V) { return sizeof(float) * (size_t)(V + 40); }          // row_topk_kernel / row_topk_thresh_kernel
+size_t sample_smem_bytes(int V) { return sizeof(float) * (size_t)(2 * V + 40); }    // row_sample_kernel
+
+// Where the vocabulary stage of a decode runs (sat_decode_vocab_path): the shared-memory row kernels when a logits row fits, the
+// fused candidate lists of the vocabulary GEMM's epilogue otherwise (or always under SAT_VOCAB_TOPK=1, for A/B timing); greedy
+// decode on the tensor cores always takes the fused arg-max.  One choice per call, so that every step reads the same buffers.
+int vocab_path(const SatDims& d, int k, int sample) {
+  const int V = d.V;
+  const bool fused_ok = d.dtype == SAT_BF16 && d.use_tc != 0 && d.exact == 0;
+  if (fused_ok && k == 1 && sample == SAT_SAMPLE_BEAM) return SAT_VOCAB_PATH_GREEDY;
+  static const int force_cand = getenv("SAT_VOCAB_TOPK") ? atoi(getenv("SAT_VOCAB_TOPK")) : 0;
+  const bool rows_fit = topk_smem_bytes(V) <= SMEM_LIMIT && (sample != SAT_SAMPLE_MULTINOMIAL || sample_smem_bytes(V) <= SMEM_LIMIT);
+  if (fused_ok && (force_cand != 0 || !rows_fit)) return SAT_VOCAB_PATH_CAND;
+  SAT_REQUIRE(topk_smem_bytes(V) <= SMEM_LIMIT, "vocabulary of %d words needs %zu bytes of shared memory per row in the top-k kernel "
+              "(limit 227 KB); decoding at this size needs the bf16 tensor-core path (bf16, use_tc, not exact)", V, topk_smem_bytes(V));
+  SAT_REQUIRE(rows_fit, "vocabulary of %d words is too large for the multinomial sampler's shared memory; decoding at this size needs "
+              "the bf16 tensor-core path (bf16, use_tc, not exact)", V);
+  return SAT_VOCAB_PATH_ROWS;
+}
+
 template <typename TS, bool kExact>
 int decode_impl(const SatDims& d, const SatWeights& w, SatDecodeBuffers& b, cudaStream_t st) {
   const int R = d.B, n_img = d.Bi, k = d.ncap, L = d.L, D = d.D, A = d.A, E = d.E, H = d.H, V = d.V;
@@ -45,17 +66,25 @@ int decode_impl(const SatDims& d, const SatWeights& w, SatDecodeBuffers& b, cuda
   SAT_LAUNCH_OK();
 
   const float scale = (float)(1.0 / sqrt((double)L));
-  const size_t topk_smem = sizeof(float) * (size_t)(V + 40);
+  const size_t topk_smem = topk_smem_bytes(V);
   const int V0 = d.V0 ? d.V0 : V;
+  const int path = vocab_path(d, k, b.sample_method);
+  if (path < 0) return path;
+  const bool fused_operands = tc::operands_ok(gemm_a1(b.xo, E, E), w.Wo, E);
   // greedy on the tensor cores: soft-max statistics and the best word come out of the vocabulary GEMM's epilogue
-  const bool fuse_greedy = k == 1 && b.topk_stats != nullptr && std::is_same<TS, bf16>::value && tc && !kExact &&
-                           b.sample_method == 0 && tc::operands_ok(gemm_a1(b.xo, E, E), w.Wo, E);
-  SAT_REQUIRE(fuse_greedy || topk_smem <= 227 * 1024, "vocabulary of %d words needs %zu bytes of shared memory per row in the top-k kernel "
-              "(limit 227 KB)", V, topk_smem);
+  const bool fuse_greedy = path == SAT_VOCAB_PATH_GREEDY && b.topk_stats != nullptr && fused_operands;
+  // beam search / sampling above the row kernels' sizes: per-tile candidate lists come out of the epilogue
+  const bool fuse_cand = path == SAT_VOCAB_PATH_CAND;
+  SAT_REQUIRE(!fuse_cand || (fused_operands && b.topk_stats && b.tile_val && b.tile_idx &&
+                             (b.sample_method != SAT_SAMPLE_MULTINOMIAL || (b.tile_key && b.topk_stats2))),
+              "sat_decode: the fused candidate path needs aligned operands and the topk_stats / tile_* buffers");
+  SAT_REQUIRE(fuse_greedy || fuse_cand || topk_smem <= SMEM_LIMIT, "vocabulary of %d words needs %zu bytes of shared memory per row in "
+              "the top-k kernel (limit 227 KB)", V, topk_smem);
+  SAT_REQUIRE(fuse_greedy || fuse_cand || b.logits != nullptr, "sat_decode: logits buffer missing");
   // candidate selection: threshold kernel (SAT_TOPK_MODE=0 forces the plain scan kernel for A/B runs)
   static const int topk_mode = getenv("SAT_TOPK_MODE") ? atoi(getenv("SAT_TOPK_MODE")) : 1;
   auto topk_k = (topk_mode == 0 || k == 1) ? row_topk_kernel : row_topk_thresh_kernel;      // greedy: one scan is already minimal
-  if (topk_smem > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(topk_k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)topk_smem));
+  if (!fuse_greedy && !fuse_cand && topk_smem > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(topk_k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)topk_smem));
   // sampling decoders (sample_method "multinomial" / "topk", model.py:360-379) and decoder noise (model.py:322-324)
   const int sample = b.sample_method;
   const int kcap = b.kcap > 0 ? b.kcap : k;
@@ -63,11 +92,9 @@ int decode_impl(const SatDims& d, const SatWeights& w, SatDecodeBuffers& b, cuda
   const bool noisy = b.decoder_noise != 0.0f;
   SAT_REQUIRE(sample == SAT_SAMPLE_BEAM || (b.cand_key != nullptr || sample == SAT_SAMPLE_TOPK), "sat_decode: cand_key buffer missing");
   SAT_REQUIRE(!noisy || b.h_noisy != nullptr, "sat_decode: h_noisy buffer missing");
-  const size_t samp_smem = sizeof(float) * (size_t)(2 * V + 40);
-  if (sample == SAT_SAMPLE_MULTINOMIAL) {
-    SAT_REQUIRE(samp_smem <= 227 * 1024, "vocabulary of %d words is too large for the multinomial sampler's shared memory", V);
-    if (samp_smem > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(row_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)samp_smem));
-  }
+  const size_t samp_smem = sample_smem_bytes(V);
+  if (sample == SAT_SAMPLE_MULTINOMIAL && !fuse_cand && samp_smem > 48 * 1024)
+    SAT_CUDA(cudaFuncSetAttribute(row_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)samp_smem));
   BeamParams bp{k, V, S, b.tokEND, b.rescore, b.reward, S + 1, kcap, sample, b.sample_topk, b.sample_seed};
   const int64_t hist_sz = (int64_t)R * (S + 1);
 
@@ -121,6 +148,23 @@ int decode_impl(const SatDims& d, const SatWeights& w, SatDecodeBuffers& b, cuda
       SAT_CUDA(sat_launch_pdl(tc::greedy_finalize_kernel, dim3((R + 7) / 8), dim3(256), 0, st, (const float4*)va.stats, va.NT,
                               (const int32_t*)b.alive, (const float*)b.top_scores, R, (int)(step == 0), b.cand_val, b.cand_idx));
       SAT_COUNT_LAUNCH();
+    } else if (fuse_cand) {
+      const bool samp = sample == SAT_SAMPLE_MULTINOMIAL && step > 0;
+      tc::VocabArgs va{};
+      va.bias = w.bo; va.V0 = V0; va.NT = (V + 127) / 128; va.stats = reinterpret_cast<float4*>(b.topk_stats);
+      va.alive = b.alive; va.inv_temp = 1.0f / b.temps[step];
+      va.tokPAD = b.tokPAD; va.tokSTART = b.tokSTART; va.tokEND = b.tokEND; va.tokUNK = b.tokUNK; va.step0 = step == 0;
+      va.kcap = kcap; va.cand_x = b.tile_val; va.cand_col = b.tile_idx; va.cand_key = b.tile_key;
+      va.stats2 = reinterpret_cast<float2*>(b.topk_stats2); va.sharp = 20.0f / (float)(step > 0 ? step : 1);
+      va.seed = b.sample_seed; va.step = step;
+      if (samp) SAT_TRY((tc::launch_vocab<tc::VOCAB_SAMPLE>(gemm_a1(b.xo, E, E), (const bf16*)w.Wo, E, R, V, va, st)));
+      else SAT_TRY((tc::launch_vocab<tc::VOCAB_TOPK>(gemm_a1(b.xo, E, E), (const bf16*)w.Wo, E, R, V, va, st)));
+      SAT_PROF(3, st);
+      SAT_CUDA(sat_launch_pdl(samp ? tc::cand_finalize_kernel<true> : tc::cand_finalize_kernel<false>, dim3((R + 7) / 8), dim3(256), 0,
+                              st, (const float4*)va.stats, (const float2*)va.stats2, (const float*)b.tile_val, (const float*)b.tile_key,
+                              (const int32_t*)b.tile_idx, va.NT, kcap, (const float*)b.top_scores, (const int32_t*)b.kcur, k,
+                              samp ? 0 : kk_req, R, (int)(step == 0), b.cand_key, b.cand_val, b.cand_idx));
+      SAT_COUNT_LAUNCH();
     } else {
       SAT_TRY((gemm_tn<TS, TS>(tc, gemm_a1(b.xo, E, E), (const TS*)w.Wo, E, R, V, EpiStore<float>{b.logits, V, w.bo, nullptr, 0}, st)));
       SAT_PROF(3, st);
@@ -169,6 +213,15 @@ int sat_decode_prepare_weights(const SatDims* d, const SatWeights* w, float* GxV
                                  EpiStore<float>{GxV, 4 * d->H, w->bg, nullptr, 0}, st);
   return gemm_tn<bf16, bf16>(tc, gemm_a1(w->Emb, d->E, d->E), (const bf16*)w->Wihe, d->E, d->V, 4 * d->H,
                              EpiStore<float>{GxV, 4 * d->H, w->bg, nullptr, 0}, st);
+}
+
+int sat_decode_vocab_path(const SatDims* d, int k, int sample_method, int sample_topk) {
+  SAT_REQUIRE(d != nullptr, "sat_decode_vocab_path: NULL dims");
+  SAT_REQUIRE(k >= 1 && k <= 32, "sat_decode_vocab_path: beam width %d outside 1..32", k);
+  SAT_REQUIRE(sample_method >= 0 && sample_method <= 2, "sat_decode_vocab_path: unknown sample_method %d", sample_method);
+  SAT_REQUIRE(sample_method != SAT_SAMPLE_TOPK || (sample_topk >= 1 && sample_topk <= 32),
+              "sat_decode_vocab_path: the topk sampler needs 1 <= sample_topk <= 32");
+  return vocab_path(*d, k, sample_method);
 }
 
 int sat_decode(const SatDims* d, const SatWeights* w, SatDecodeBuffers* b, void* stream) {

@@ -262,12 +262,6 @@ row_topk_thresh_kernel(const float* __restrict__ logits, const float* __restrict
 // word), so a decode is reproducible under its seed; it is not the reference's torch RNG stream (not parity-checkable).
 enum { SAT_SAMPLE_BEAM = 0, SAT_SAMPLE_MULTINOMIAL = 1, SAT_SAMPLE_TOPK = 2 };
 
-__device__ __forceinline__ float sat_uniform01(uint64_t seed, uint32_t stream, uint64_t idx) {      // in (0, 1)
-  return ((float)(sat_hash32(seed, stream, idx) >> 8) + 0.5f) * (1.0f / 16777216.0f);
-}
-__device__ __forceinline__ float sat_gumbel(uint64_t seed, uint32_t stream, uint64_t idx) {
-  return -logf(-logf(sat_uniform01(seed, stream, idx)));
-}
 
 // sample_method = "multinomial" (model.py:360-364), steps > 0: the reference draws kc flat indices from
 // softmax(20 * seq_scores / step, dim=1).reshape(-1).  Per row: key_v = y_v - logsumexp(y) + Gumbel, y = 20 * log_softmax(x)_v / step

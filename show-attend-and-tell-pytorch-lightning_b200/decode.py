@@ -58,8 +58,10 @@ def decode_annotations(dw, ann_bld, k, max_gen_length, temperature=1.0, rescore_
     kcap = max(k, int(sample_topk)) if method == 2 else k
     if (method != 0 or noise != 0.0) and seed is None:
         seed = int(torch.randint(0, 2 ** 62, (1,)).item())
-    # greedy on the tensor cores: per-tile soft-max statistics replace the [R,V] logits
-    fuse_greedy = k == 1 and method == 0 and dw.use_tc and dtype == torch.bfloat16 and not dw.exact
+    # which vocabulary stage runs (row kernels on [R,V] logits, or per-tile statistics / candidates from the GEMM epilogue)
+    path = L_.sat_decode_vocab_path(C.byref(d), k, method, int(sample_topk))
+    if path < 0:
+        _lib.check(path, "sat_decode")
     f, s, i32 = torch.float32, dtype, torch.int32
     _n = [0]
 
@@ -81,10 +83,15 @@ def decode_annotations(dw, ann_bld, k, max_gen_length, temperature=1.0, rescore_
         t["cand_key"] = mk((R, kcap), f)
     if noise != 0.0:
         t["h_noisy"] = mk((nl, R, H), s)
-    if fuse_greedy:
-        t["topk_stats"] = mk((R, (V + 127) // 128, 4), f)
-    else:
+    NT = (V + 127) // 128
+    if path == _lib.VOCAB_PATH_ROWS:
         t["logits"] = mk((R, V), f)
+    else:
+        t["topk_stats"] = mk((R, NT, 4), f)
+    if path == _lib.VOCAB_PATH_CAND:
+        t["tile_val"], t["tile_idx"] = mk((R, NT, kcap), f), mk((R, NT, kcap), i32)
+        if method == 1:
+            t["tile_key"], t["topk_stats2"] = mk((R, NT, kcap), f), mk((R, NT, 2), f)
     temps = temperature if isinstance(temperature, (list, tuple)) else [temperature]
     temps_arr = (C.c_float * (S + 1))(*[float(temps[i % len(temps)]) for i in range(S + 1)])
     b = _lib.SatDecodeBuffers()
