@@ -121,7 +121,9 @@ typedef struct SatTrainBuffers {
   const int32_t* caps;   /* [B,T+1]      encoded captions, column 0 = <START>                     */
   const int32_t* lens;   /* [B]          number of targets per caption (model.py:492)             */
   const int32_t* sampled; /* HOST pointer, [T] flags or NULL: step t feeds back argmax_v logits[t-1] instead of the ground-truth
-                            word (scheduled sampling, model.py:518-523; the host draws torch.rand(1) per step > 2)      */
+                            word (scheduled sampling, model.py:518-523; the host draws torch.rand(1) per step > 2); on the fused
+                            path a caption finished before step t-1 keeps its ground-truth word.  sat_train_vocab_path(d, 1) names the
+                            vocabulary path, and so the buffers, such a call needs                                         */
   /* fwd */
   int32_t* tok;          /* [T,B]        previous-word ids actually fed at each step (ground truth or sampled)      */
   void* P;               /* [Bi,L,A] s   W_a * a, once per image (reference recomputes per step, model.py:100) */
@@ -326,6 +328,18 @@ int sat_resize_nhwc_fwd(const void* src, void* dst, int32_t n, int32_t h, int32_
                         void* stream);
 int sat_resize_nhwc_bwd(const void* d_dst, void* d_src, int32_t n, int32_t h, int32_t w, int32_t H2, int32_t W2, int32_t D, int32_t dtype,
                         void* stream);
+
+/* Which vocabulary stage sat_train_forward runs for these dims, teacher-forced (sampled = 0) or with scheduled-sampling steps
+ * (sampled != 0), and so which buffers it reads: SAT_TRAIN_PATH_LOGITS = [T,B,V] `logits` + the shared-memory cross-entropy row
+ * kernel (V <= 58,072), SAT_TRAIN_PATH_FUSED = `ce_stats` / `row_lse` / `row_xt` (+ `dlogits` with backward), no logits: the
+ * vocabulary GEMM's epilogue keeps per-tile statistics, and a sampled step feeds back the arg-max read from them.  Teacher-forced:
+ * FUSED wherever it can run (bf16 tensor cores; the caller may still keep the logits instead).  Sampled, bf16 tensor cores: FUSED
+ * where a logits row does not fit the row kernel, or everywhere under SAT_TRAIN_FUSED_SS=1; LOGITS otherwise.  A caller that
+ * wants the logits back (train_batch) passes `logits` and no `ce_stats`, and is held to the row kernel's limit.  < 0 (error
+ * set) when no path takes the call (fp32, or bf16 without tensor cores, above the limit). */
+#define SAT_TRAIN_PATH_LOGITS 0
+#define SAT_TRAIN_PATH_FUSED 1
+int sat_train_vocab_path(const SatDims* d, int32_t sampled);
 
 int sat_train_forward(const SatDims* d, const SatWeights* w, SatTrainBuffers* b, void* stream);
 

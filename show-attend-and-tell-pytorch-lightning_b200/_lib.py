@@ -70,8 +70,10 @@ class SatParamGrads(C.Structure):
 EXPORTS = ["sat_version", "sat_last_error", "sat_abi_sizeof", "sat_launch_count", "sat_profile_begin", "sat_profile_end", "sat_dropout_multiplier", "sat_pack_weights",
            "sat_linear", "sat_linear_nt", "sat_prepare_images", "sat_resize_nhwc_fwd", "sat_resize_nhwc_bwd",
            "sat_attention_step_fwd", "sat_cast_captions", "sat_train_forward", "sat_train_backward", "sat_param_grads_workspace_bytes", "sat_train_param_grads",
+           "sat_train_vocab_path",
            "sat_decode_prepare_weights", "sat_decode", "sat_decode_vocab_path"]
 VOCAB_PATH_ROWS, VOCAB_PATH_GREEDY, VOCAB_PATH_CAND = 0, 1, 2      # sat_decode_vocab_path
+TRAIN_PATH_LOGITS, TRAIN_PATH_FUSED = 0, 1                           # sat_train_vocab_path
 
 _lib = None
 
@@ -121,6 +123,7 @@ def lib():
     L.sat_resize_nhwc_bwd.argtypes = [vp, vp] + [C.c_int32] * 7 + [vp]
     L.sat_cast_captions.argtypes = [vp, vp, vp, vp, C.c_int64, C.c_int64, vp]
     L.sat_train_forward.argtypes = [C.POINTER(SatDims), C.POINTER(SatWeights), C.POINTER(SatTrainBuffers), vp]
+    L.sat_train_vocab_path.argtypes = [C.POINTER(SatDims), C.c_int32]
     L.sat_train_backward.argtypes = [C.POINTER(SatDims), C.POINTER(SatWeights), C.POINTER(SatTrainBuffers), vp]
     L.sat_param_grads_workspace_bytes.argtypes = [C.POINTER(SatDims)]
     L.sat_param_grads_workspace_bytes.restype = C.c_int64

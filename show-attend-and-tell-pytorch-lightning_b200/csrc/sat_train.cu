@@ -9,7 +9,9 @@
 //  * the recurrent part of a step is three launches: h-projection GEMM (q | beta_pre | W_hh h),
 //    fused attention kernel, gate GEMM with the LSTM cell in its epilogue;
 //  * finished captions are predicated (t < lens[b]) instead of compacted, so there is no host
-//    sync, no gather/scatter of state and no per-step reallocation.
+//    sync, no gather/scatter of state and no per-step reallocation;
+//  * a scheduled-sampling step t (model.py:518-523) computes step t-1's output rows inside the loop: deep output, then
+//    either the logits + row_argmax_kernel or, on the fused path, the VOCAB_STATS tiles + ss_feedback_kernel (no logits).
 #include "sat_gemm.cuh"
 #include "sat_attention_pipe.cuh"
 #include "sat_kernels.cuh"
@@ -55,6 +57,24 @@ static int prepare_images_impl(const SatDims& d, const SatWeights& w, const void
   return 0;
 }
 
+constexpr size_t CE_SMEM_LIMIT = 227 * 1024;
+size_t ce_smem_bytes(int V) { return sizeof(float) * (size_t)(V + 40); }      // ce_rows_kernel: one logits row + scratch
+
+// Where the vocabulary stage of a training step runs (sat_train_vocab_path): 1 = fused (VOCAB_STATS / VOCAB_DLOGITS in the
+// vocabulary GEMM's epilogue, no logits), 0 = logits + ce_rows_kernel.  Teacher-forced steps: the fused path wherever it can
+// run (bf16 tensor cores), and the caller decides whether it keeps the logits instead.  Scheduled sampling: the unfused path
+// while ce_rows_kernel holds a logits row, the fused one beyond that, or wherever it can run under SAT_TRAIN_FUSED_SS=1 (A/B
+// timing, equivalence tests).  An error when the vocabulary fits neither.
+int train_vocab_path(const SatDims& d, bool sampled) {
+  const bool fused_ok = d.dtype == SAT_BF16 && d.use_tc != 0 && d.exact == 0;
+  const bool rows_fit = ce_smem_bytes(d.V) <= CE_SMEM_LIMIT;
+  static const int force_fused = getenv("SAT_TRAIN_FUSED_SS") ? atoi(getenv("SAT_TRAIN_FUSED_SS")) : 0;
+  if (fused_ok && (!sampled || !rows_fit || force_fused != 0)) return SAT_TRAIN_PATH_FUSED;
+  SAT_REQUIRE(rows_fit, "vocabulary of %d words needs %zu bytes of shared memory per row in the unfused cross-entropy kernel "
+              "(limit 227 KB); training at this size needs the bf16 tensor-core path (bf16, use_tc, not exact)", d.V, ce_smem_bytes(d.V));
+  return SAT_TRAIN_PATH_LOGITS;
+}
+
 template <typename TS, bool kExact>
 int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b, cudaStream_t st) {
   const int B = d.B, Bi = d.Bi, L = d.L, D = d.D, A = d.A, E = d.E, H = d.H, V = d.V, T = d.T;
@@ -65,8 +85,19 @@ int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b
   const TS* ann = (const TS*)b.ann;
   // fused vocabulary projection + cross entropy (tensor-core mode): the logits are never written
   const bool fuse_ce = b.ce_stats != nullptr && b.row_lse != nullptr && b.row_xt != nullptr && std::is_same<TS, bf16>::value && tc && !kExact &&
-                       b.sampled == nullptr && tc::operands_ok(gemm_a1(b.Xo, E, E), w.Wo, E);
+                       tc::operands_ok(gemm_a1(b.Xo, E, E), w.Wo, E);
   SAT_REQUIRE(fuse_ce || b.logits != nullptr, "sat_train_forward: logits buffer missing (only the fused tensor-core path can do without)");
+  if (b.sampled != nullptr) {
+    // scheduled sampling: sat_train_vocab_path decides; a caller that asks for the logits (train_batch) always gets them
+    const int path = train_vocab_path(d, true);
+    if (path < 0) return path;
+    SAT_REQUIRE(!fuse_ce || path == SAT_TRAIN_PATH_FUSED, "sat_train_forward: fused vocabulary buffers given to a scheduled-sampling step whose "
+                "vocabulary path is the unfused one (sat_train_vocab_path)");
+  }
+  SAT_REQUIRE(fuse_ce || ce_smem_bytes(V) <= CE_SMEM_LIMIT, "vocabulary of %d words needs %zu bytes of shared memory per row in the "
+              "unfused cross-entropy kernel (limit 227 KB); training at this size needs the bf16 tensor-core path (bf16, use_tc, "
+              "not exact) without kept logits", V, ce_smem_bytes(V));
+  const int NTv = (V + 127) / 128;                        // 128-column vocabulary tiles per row (fused path)
 
   // ---- once per image ------------------------------------------------------------------------
   const int nl = d.layers > 1 ? d.layers : 1;
@@ -101,9 +132,19 @@ int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b
       // scheduled sampling (model.py:518-523): this step's input word is argmax_v logits[t-1]; compute the output of
       // step t-1 now (the hoisted whole-sequence GEMMs below recompute the same values), then re-embed and re-project.
       const int64_t o1 = (int64_t)(t - 1) * B;
+      SAT_PROF(8, st);                                      // 8 = the extra work of a sampled step, deep output to Gx[t]
       SAT_TRY((gemm_tn<TS, TS>(tc, gemm_a2((const TS*)Hs_top + (int64_t)t * B * H, H, H, (const TS*)b.Z + o1 * D, D, D), (const TS*)w.Whozo,
                                H + D, B, E, EpiTanhAdd<TS, kExact>{(const TS*)b.Xe + o1 * E, (TS*)b.Xo + o1 * E, E, nullptr, d.plain_output, b.dropout_p, b.dropout_seed, o1}, st)));
-      if (b.logits_f32) {
+      if (fuse_ce) {
+        // fused: the tile statistics of step t-1's rows (the hoisted pass rewrites them with the same values), then the
+        // arg-max of each live row by the rule ce_finalize_kernel reports as row_argmax; no logits are written
+        tc::VocabArgs va{};
+        va.bias = w.bo; va.V0 = V0; va.NT = NTv; va.stats = reinterpret_cast<float4*>(b.ce_stats) + o1 * NTv;
+        va.caps = b.caps; va.lens = b.lens; va.B = B; va.caplen = caplen; va.row0 = (int)o1; va.row_xt = b.row_xt + o1;
+        SAT_TRY((tc::launch_vocab<tc::VOCAB_STATS>(gemm_a1((const TS*)b.Xo + o1 * E, E, E), (const bf16*)w.Wo, E, B, V, va, st)));
+        SAT_CUDA(sat_launch_pdl(tc::ss_feedback_kernel, dim3((B + 7) / 8), dim3(256), 0, st, (const float4*)va.stats, NTv,
+                                (const int32_t*)b.lens, B, t, V0, b.tok + (int64_t)t * B));
+      } else if (b.logits_f32) {
         SAT_TRY((gemm_tn<TS, TS>(tc, gemm_a1((const TS*)b.Xo + o1 * E, E, E), (const TS*)w.Wo, E, B, V,
                                  EpiStore<float>{(float*)b.logits + o1 * V, V, w.bo, nullptr, 0}, st)));
         row_argmax_kernel<float><<<B, 256, 0, st>>>((const float*)b.logits + o1 * V, b.tok + (int64_t)t * B, V);
@@ -119,6 +160,7 @@ int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b
       SAT_LAUNCH_OK();
       SAT_TRY((gemm_tn<TS, TS>(tc, gemm_a1((const TS*)b.Xe + (int64_t)t * B * E, E, E), (const TS*)w.Wihe, E, B, 4 * H,
                                EpiStore<float>{b.Gx + (int64_t)t * B * 4 * H, 4 * H, w.bg, nullptr, 0}, st)));
+      SAT_PROF(8, st);
     }
     const TS* h_t = (const TS*)b.Hs + (int64_t)t * B * H;            // layer 0
     const float* c_t = b.Cs + (int64_t)t * B * H;
@@ -172,7 +214,7 @@ int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b
     // pass 1: per-tile soft-max statistics in the GEMM epilogue; finish per row; pass 2 (training only): recompute the tiles
     // into dlogits.  HBM traffic of the stage: one bf16 [T*B, V] write instead of write + read + write.
     tc::VocabArgs va{};
-    va.bias = w.bo; va.V0 = V0; va.NT = (V + 127) / 128; va.stats = reinterpret_cast<float4*>(b.ce_stats);
+    va.bias = w.bo; va.V0 = V0; va.NT = NTv; va.stats = reinterpret_cast<float4*>(b.ce_stats);
     va.caps = b.caps; va.lens = b.lens; va.B = B; va.caplen = caplen; va.row_xt = b.row_xt; va.row_lse = b.row_lse;
     va.inv_ntok_p = b.out + 4; va.smoothing = b.label_smoothing; va.dlogits = (bf16*)b.dlogits; va.ldd = V;
     SAT_TRY((tc::launch_vocab<tc::VOCAB_STATS>(gemm_a1(b.Xo, E, E), (const bf16*)w.Wo, E, T * B, V, va, st)));
@@ -191,9 +233,7 @@ int train_forward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& b
     }
     SAT_PROF(3, st);
     // ---- loss ----------------------------------------------------------------------------------
-    const size_t ce_smem = sizeof(float) * (size_t)(V + 40);
-    SAT_REQUIRE(ce_smem <= 227 * 1024, "vocabulary of %d words needs %zu bytes of shared memory per row in the unfused cross-entropy "
-                "kernel (limit 227 KB): use the fused tensor-core path (bf16) for vocabularies this large", V, ce_smem);
+    const size_t ce_smem = ce_smem_bytes(V);              // within the limit: checked before the first launch
     if (b.logits_f32) {
       auto k = ce_rows_kernel<float, TS, kExact>;
       if (ce_smem > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ce_smem));
@@ -299,6 +339,11 @@ int sat_cast_captions(const int64_t* caps64, const int64_t* lens64, int32_t* cap
   SAT_COUNT_LAUNCH();
   SAT_LAUNCH_OK();
   return 0;
+}
+
+int sat_train_vocab_path(const SatDims* d, int32_t sampled) {
+  SAT_TRY(check_dims(d));
+  return train_vocab_path(*d, sampled != 0);
 }
 
 int sat_train_forward(const SatDims* d, const SatWeights* w, SatTrainBuffers* b, void* stream) {

@@ -3,6 +3,8 @@
 // of the tcgen05 GEMM core (sat_gemm_tc.cuh).  The [T*B, V] logits never reach HBM:
 //   pass 1 (VOCAB_STATS)   per (row, 128-column tile): max, sum exp(x - max), sum x, arg-max, and the target logit
 //   ce_finalize_kernel     per row: log-sum-exp, token loss, arg-max
+//   ss_feedback_kernel     scheduled sampling: pass 1 over one step's B rows inside the time loop, then the arg-max of each row
+//                          becomes the next step's input word (the same rule as ce_finalize_kernel's arg-max)
 //   pass 2 (VOCAB_DLOGITS) recomputes the tile and writes dlogits = (softmax - target distribution) / N_tok in the operand
 //                          dtype -- the only [T*B, V] array of the training step (it feeds dpre = dlogits * Wo and dWo)
 //   VOCAB_GREEDY           per (row, tile): soft-max statistics of x / temperature and the best non-masked word;
@@ -39,6 +41,7 @@ struct VocabArgs {
   const int32_t* caps;
   const int32_t* lens;
   int B, caplen;
+  int row0;                 // time-major row of the launch's first row (0: whole sequence; (t-1)*B: one step of scheduled sampling)
   float* row_xt;            // [M] logit of the target word (written by the one thread that owns its column)
   const float* row_lse;     // [M]                                     (DLOGITS)
   const float* inv_ntok_p;  //                                         (DLOGITS)
@@ -97,7 +100,7 @@ struct EpiVocab {
     if (MODE == VOCAB_GREEDY) {
       active = active && a.alive[m] != 0;
     } else {
-      const int t = m / a.B, b = m - t * a.B;
+      const int mg = a.row0 + m, t = mg / a.B, b = mg - t * a.B;
       active = active && t < a.lens[b];
       if (active) y = a.caps[(int64_t)b * a.caplen + t + 1];
     }
@@ -413,6 +416,25 @@ struct EpiVocab {
   }
 };
 
+// Arg-max of a row over its VOCAB_STATS tiles, the first maximal word (torch.argmax): a tile's max is the value of its arg-max
+// and tiles ascend with the columns.  Warp-collective; every lane returns the row's (max, arg-max).  The one rule for both the
+// reported arg-max (ce_finalize_kernel) and the word scheduled sampling feeds back (ss_feedback_kernel).
+__device__ __forceinline__ int tiles_argmax(const float4* __restrict__ st, int NT, int lane, float& mx_out) {
+  float mx = -INFINITY;
+  int arg = 0x7fffffff;
+  for (int i = lane; i < NT; i += 32) {
+    const float4 s4 = st[i];
+    if (s4.x > mx) { mx = s4.x; arg = __float_as_int(s4.w); }
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
+    if (om > mx || (om == mx && oa < arg)) { mx = om; arg = oa; }
+  }
+  mx_out = mx;
+  return arg;
+}
+
 // Row-wise finish of the fused cross entropy: log-sum-exp over the tile statistics, token loss (util.py:105-112) and arg-max
 // (model.py:596).  One warp per row, fixed combination order.
 static __global__ void __launch_bounds__(256)
@@ -429,17 +451,8 @@ ce_finalize_kernel(const float4* __restrict__ stats, int NT, const float* __rest
     return;
   }
   const float4* st = stats + (int64_t)m * NT;
-  float mx = -INFINITY;
-  int arg = 0x7fffffff;
-  for (int i = lane; i < NT; i += 32) {
-    const float4 s4 = st[i];
-    if (s4.x > mx) { mx = s4.x; arg = __float_as_int(s4.w); }      // a tile's max is the value of its arg-max; tiles ascend
-  }
-  for (int o = 16; o > 0; o >>= 1) {
-    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
-    const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
-    if (om > mx || (om == mx && oa < arg)) { mx = om; arg = oa; }
-  }
+  float mx;
+  const int arg = tiles_argmax(st, NT, lane, mx);
   float se = 0.0f, sx = 0.0f;
   for (int i = lane; i < NT; i += 32) {
     const float4 s4 = st[i];
@@ -456,6 +469,22 @@ ce_finalize_kernel(const float4* __restrict__ stats, int NT, const float* __rest
     row_loss[m] = (1.0f - smoothing) * nll + smoothing * smooth;
     row_argmax[m] = arg;
   }
+}
+
+// Scheduled sampling on the fused path (model.py:518-523): the word fed at step t is the arg-max of step t-1's logits, read from
+// the VOCAB_STATS tiles of those B rows (stats = [B][NT] of step t-1).  A caption finished at step t-1 (t-1 >= lens[b])
+// keeps its teacher-forced word (it only has to be a valid id: nothing reads that row's outputs).  A row without a finite maximum
+// (non-finite logits) is fed <PAD>, as row_argmax_kernel does; the bad-id flag out[6] belongs to the captions and is left alone.
+static __global__ void __launch_bounds__(256)
+ss_feedback_kernel(const float4* __restrict__ stats, int NT, const int32_t* __restrict__ lens, int B, int t, int V0,
+                   int32_t* __restrict__ tok_t) {
+  SAT_PDL_TRIGGER();
+  SAT_PDL_WAIT();
+  const int lane = threadIdx.x & 31, b = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (b >= B || t - 1 >= lens[b]) return;
+  float mx;
+  const int arg = tiles_argmax(stats + (int64_t)b * NT, NT, lane, mx);
+  if (lane == 0) tok_t[b] = (unsigned)arg < (unsigned)V0 ? arg : 0;
 }
 
 // Greedy decode: candidate (score, word) of every live row from the tile statistics -- the k = 1 output of

@@ -155,12 +155,26 @@ def annotations_as_bld(ann, dtype, D_storage=None):
     return x.contiguous()
 
 
+def vocab_path_fused(d, sampled=None, fuse_ce=True):
+    """Whether sat_train_forward runs the vocabulary stage fused (per-tile statistics in the GEMM epilogue, no [T,B,V] logits):
+    sat_train_vocab_path decides.  Teacher-forced: fused when the caller asks for it (fuse_ce) and the library can run it.
+    Scheduled sampling: the library's choice (the logits path while the cross-entropy row kernel holds a row, the fused path
+    above that); a caller that wants the logits back passes fuse_ce=False and is held to the row kernel's limit.  Raises
+    SatError when neither path can run these dims."""
+    is_sampled = sampled is not None and any(sampled)
+    path = _lib.lib().sat_train_vocab_path(C.byref(d), 1 if is_sampled else 0)
+    if path < 0:
+        _lib.check(path, "sat_train_vocab_path")
+    return bool(fuse_ce) and path == _lib.TRAIN_PATH_FUSED
+
+
 def train_forward(pw, ann_bld, caps, lens, label_smoothing=0.0, att_gamma=1.0, exact=True, use_tc=False,
                   logits_f32=False, backward=True, keep_logits=False, buffers=None, sampled=None, dropout=(0.0, 0.0, 0),
                   fuse_ce=False):
     """ann_bld [Bi,L,D] (pw.dtype, cuda); caps [Bi,ncap,T+1] or [B,T+1] int; lens [Bi,ncap] or [B].
     Runs sat_train_forward; returns the TrainBuffers (loss etc. in .t['out']).  fuse_ce=True (tensor-core mode) keeps the
-    vocabulary logits on chip: .t has no 'logits' then."""
+    vocabulary logits on chip: .t has no 'logits' then.  With scheduled-sampling steps (sampled) the library picks the path
+    (vocab_path_fused); keep_logits / logits_f32 always keep the logits."""
     L_ = _lib.lib()
     dev = ann_bld.device
     Bi, L, D = ann_bld.shape
@@ -184,8 +198,7 @@ def train_forward(pw, ann_bld, caps, lens, label_smoothing=0.0, att_gamma=1.0, e
     assert D == dm["D"], "annotation width %d != encoder_dim %d" % (D, dm0["D"])
     assert ann_bld.dtype == pw.dtype and ann_bld.is_contiguous()
     d = make_dims(B, Bi, L, pw, caplen - 1, pw.dtype, exact, use_tc)
-    if sampled is not None and any(sampled):
-        fuse_ce = False                     # scheduled sampling feeds arg-max(logits[t-1]) back: per-step logits are needed
+    fuse_ce = vocab_path_fused(d, sampled, fuse_ce and not (keep_logits or logits_f32))
     if buffers is None:
         buffers = TrainBuffers(d, pw.dtype, dev, logits_f32=logits_f32, backward=backward, keep_logits=keep_logits, fuse_ce=fuse_ce)
     buffers.bind_inputs(ann_bld, caps2, lens2, label_smoothing, att_gamma, sampled, dropout)
