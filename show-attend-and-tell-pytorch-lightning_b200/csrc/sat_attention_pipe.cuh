@@ -63,7 +63,14 @@ constexpr int ATTP_BWD_CW = 8;                       // backward: with the dP ac
 constexpr int ATTP_NST = 6;
 constexpr int ATTP_STAGE_BYTES = 16384;
 constexpr size_t SAT_ATT_GROUP_MIN_BYTES = 0;   // per-image annotation tile from which the grouped kernel is used (measured faster at every size tried)
-constexpr int ATTP_KA = 2;                           // attention_dim <= 256 on the pipelined kernel
+// Attention columns: a lane owns columns lane*4 + 128*k, k < KA, so a kernel instantiated for KA serves attention_dim
+// <= 128*KA.  KA = 2 (A <= 256) keeps q and w_f in registers (ATTP_REG_KA); KA = 4 / 8 (A <= 512 / 1024) read them from
+// shared memory, where a register copy would cost 8*KA registers per lane.
+constexpr int ATTP_REG_KA = 2;
+constexpr int ATTP_MAXKA = 8;                        // attention_dim <= 1024 on the pipelined kernels
+constexpr int ATTC_MAXA = 256;                       // the opt-in 2-CTA pair kernel: attention_dim <= 256
+static inline int attp_ka(int A) { return A <= 256 ? 2 : (A <= 512 ? 4 : 8); }
+constexpr size_t ATTP_SMEM_MAX = 227 * 1024;         // opt-in dynamic shared memory per block (sm_100)
 
 struct AttPipeSmem {
   uint64_t full[ATTP_NST];
@@ -72,7 +79,66 @@ struct AttPipeSmem {
   float red_b[ATTP_MAXCW];
 };
 
-template <typename T, bool kExact, int CW>
+// KA > 2: scores of the rows l0 .. l0+3 of a P stage against one caption row, q and w_f read from shared memory (16-byte
+// loads; A % 4 == 0).  Per lane the sum runs over the column slices in order and then over the 4 columns of a slice, as
+// in the register path of the KA = 2 kernels.
+template <typename T, bool kExact, int KA>
+__device__ __forceinline__ void attp_scores4_smem(const T* Ps, int l0, int rows, int A, int lane, const float* q, const float* w,
+                                                  float s4[4]) {
+#pragma unroll 2
+  for (int k = 0; k < KA; ++k) {
+    const int a = lane * 4 + 128 * k;
+    if (a < A) {
+      float4 p[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+        p[u] = (l0 + u) < rows ? ld4(Ps + (size_t)(l0 + u) * A + a) : make_float4(0.f, 0.f, 0.f, 0.f);
+      const float4 q4 = *reinterpret_cast<const float4*>(q + a);
+      const float4 w4 = *reinterpret_cast<const float4*>(w + a);
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        s4[u] = fmaf(w4.x, sat_tanh<kExact>(p[u].x + q4.x), s4[u]);
+        s4[u] = fmaf(w4.y, sat_tanh<kExact>(p[u].y + q4.y), s4[u]);
+        s4[u] = fmaf(w4.z, sat_tanh<kExact>(p[u].z + q4.z), s4[u]);
+        s4[u] = fmaf(w4.w, sat_tanh<kExact>(p[u].w + q4.w), s4[u]);
+      }
+    }
+  }
+}
+
+// KA > 2: first 4-row group of P stage i that warp `warp` scores.  A stage holds 16 KB / (A * sizeof(T)) rows, only 4 to 16
+// at A > 256, so the groups are dealt round-robin over the warps across stages (all warps work while several stages are
+// in flight) instead of every stage starting at warp 0.  Each row is still scored by one warp.
+template <int CW>
+__device__ __forceinline__ int attp_first_row(int warp, int i, int RCP) {
+  const int ngr = (RCP + 3) / 4;
+  return 4 * (((warp - (int)(((int64_t)i * ngr) % CW)) + CW) % CW);
+}
+
+// KA > 2, grouped kernels: the scores of every active caption row of the image for the rows of one P stage
+template <typename T, bool kExact, int KA, int CW>
+__device__ __forceinline__ void attp_group_stage_scores(const T* Ps, int i, int RCP, int r0, int rows, int A, int lane, int warp,
+                                                        int ncap, unsigned act, const float* qs, const float* ws, float* e, int L4,
+                                                        float scale) {
+  for (int l0 = attp_first_row<CW>(warp, i, RCP); l0 < rows; l0 += CW * 4) {
+    for (int g = 0; g < ncap; ++g) {
+      if (!(act & (1u << g))) continue;
+      float s4[4] = {0.f, 0.f, 0.f, 0.f};
+      attp_scores4_smem<T, kExact, KA>(Ps, l0, rows, A, lane, qs + g * A, ws, s4);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) s4[u] += __shfl_xor_sync(0xffffffffu, s4[u], o);
+      }
+      if (lane < 4 && (l0 + lane) < rows) {
+        const float sv = lane == 0 ? s4[0] : (lane == 1 ? s4[1] : (lane == 2 ? s4[2] : s4[3]));
+        e[g * L4 + r0 + l0 + lane] = sv * scale;
+      }
+    }
+  }
+}
+
+template <typename T, bool kExact, int CW, int KA = ATTP_REG_KA>
 __global__ void __launch_bounds__(CW * 32 + 32)
 attention_step_fwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ P, const float* __restrict__ wf,
                                const float* __restrict__ hp, int64_t ldhp, const int32_t* __restrict__ lens, int t, int ncap,
@@ -176,15 +242,17 @@ attention_step_fwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
     const int d = tid + i * ATTP_CONSUMERS;
     bpre[i] = d < D ? hp_b[A + d] : 0.0f;
   }
-  // lane-resident slices of q and w_f: lane owns attention columns lane*4 + 128*k .. +3  (A <= 128 * ATTP_KA)
-  float qreg[ATTP_KA][4], wreg[ATTP_KA][4];
+  // lane-resident slices of q and w_f: lane owns attention columns lane*4 + 128*k .. +3  (A <= 128 * ATTP_REG_KA)
+  float qreg[ATTP_REG_KA][4], wreg[ATTP_REG_KA][4];
+  if constexpr (KA == ATTP_REG_KA) {
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
-    const int a = lane * 4 + 128 * k;
+    for (int k = 0; k < ATTP_REG_KA; ++k) {
+      const int a = lane * 4 + 128 * k;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      qreg[k][i] = a < A ? qs[a + i] : 0.0f;
-      wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+      for (int i = 0; i < 4; ++i) {
+        qreg[k][i] = a < A ? qs[a + i] : 0.0f;
+        wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+      }
     }
   }
   int it = 0;   // running chunk index (same sequence as the producer)
@@ -193,22 +261,27 @@ attention_step_fwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
     sat_mbar_wait(&hd->full[st], (uint32_t)(it / ATTP_NST) & 1u);
     const T* Ps = reinterpret_cast<const T*>(stages + (size_t)st * ATTP_STAGE_BYTES);
     const int r0 = i * RCP, rows = min(RCP, L - r0);
-    for (int l0 = warp * 4; l0 < rows; l0 += ATTP_CWARPS * 4) {     // 4 rows in flight per warp: independent chains
+    const int lfirst = KA == ATTP_REG_KA ? warp * 4 : attp_first_row<CW>(warp, i, RCP);
+    for (int l0 = lfirst; l0 < rows; l0 += ATTP_CWARPS * 4) {     // 4 rows in flight per warp: independent chains
       float s4[4] = {0.f, 0.f, 0.f, 0.f};
+      if constexpr (KA != ATTP_REG_KA) {
+        attp_scores4_smem<T, kExact, KA>(Ps, l0, rows, A, lane, qs, ws, s4);
+      } else {
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
-        const int a = lane * 4 + 128 * k;
-        if (a < A) {
-          float4 p[4];
+        for (int k = 0; k < ATTP_REG_KA; ++k) {
+          const int a = lane * 4 + 128 * k;
+          if (a < A) {
+            float4 p[4];
 #pragma unroll
-          for (int u = 0; u < 4; ++u)
-            p[u] = (l0 + u) < rows ? ld4(Ps + (size_t)(l0 + u) * A + a) : make_float4(0.f, 0.f, 0.f, 0.f);
+            for (int u = 0; u < 4; ++u)
+              p[u] = (l0 + u) < rows ? ld4(Ps + (size_t)(l0 + u) * A + a) : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
-          for (int u = 0; u < 4; ++u) {
-            s4[u] = fmaf(wreg[k][0], sat_tanh<kExact>(p[u].x + qreg[k][0]), s4[u]);
-            s4[u] = fmaf(wreg[k][1], sat_tanh<kExact>(p[u].y + qreg[k][1]), s4[u]);
-            s4[u] = fmaf(wreg[k][2], sat_tanh<kExact>(p[u].z + qreg[k][2]), s4[u]);
-            s4[u] = fmaf(wreg[k][3], sat_tanh<kExact>(p[u].w + qreg[k][3]), s4[u]);
+            for (int u = 0; u < 4; ++u) {
+              s4[u] = fmaf(wreg[k][0], sat_tanh<kExact>(p[u].x + qreg[k][0]), s4[u]);
+              s4[u] = fmaf(wreg[k][1], sat_tanh<kExact>(p[u].y + qreg[k][1]), s4[u]);
+              s4[u] = fmaf(wreg[k][2], sat_tanh<kExact>(p[u].z + qreg[k][2]), s4[u]);
+              s4[u] = fmaf(wreg[k][3], sat_tanh<kExact>(p[u].w + qreg[k][3]), s4[u]);
+            }
           }
         }
       }
@@ -329,8 +402,8 @@ attention_step_fwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
 // attention_step_fwd_pipe_kernel, so both kernels give bit-identical alpha / z / gz.
 //   smem: e[G][L4], q[G][A], w[A], ring; the cross-row-group reduction scratch red[G][RG*D] aliases the drained ring.
 // =============================================================================================
-template <typename T, bool kExact, int CW, int G>
-__global__ void __launch_bounds__(CW * 32 + 32, 2)
+template <typename T, bool kExact, int CW, int G, int KA = ATTP_REG_KA>
+__global__ void __launch_bounds__(CW * 32 + 32, KA == ATTP_REG_KA ? 2 : 1)
 attention_step_fwd_group_kernel(const T* __restrict__ ann, const T* __restrict__ P, const float* __restrict__ wf,
                                 const float* __restrict__ hp, int64_t ldhp, const int32_t* __restrict__ lens, int t, int ncap,
                                 int L, int D, int A, float scale, float* __restrict__ alpha, int64_t ld_alpha,
@@ -424,12 +497,14 @@ attention_step_fwd_group_kernel(const T* __restrict__ ann, const T* __restrict__
   for (int a = tid; a < A; a += ATTP_CONSUMERS) ws[a] = wf[a];
   sat_named_bar(1, ATTP_CONSUMERS);
 
-  float wreg[ATTP_KA][4];
+  float wreg[ATTP_REG_KA][4];
+  if constexpr (KA == ATTP_REG_KA) {
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
-    const int a = lane * 4 + 128 * k;
+    for (int k = 0; k < ATTP_REG_KA; ++k) {
+      const int a = lane * 4 + 128 * k;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+      for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+    }
   }
   int it = 0;
   for (int i = 0; i < nP; ++i, ++it) {
@@ -437,10 +512,13 @@ attention_step_fwd_group_kernel(const T* __restrict__ ann, const T* __restrict__
     sat_mbar_wait(&hd->full[st], (uint32_t)(it / ATTP_NST) & 1u);
     const T* Ps = reinterpret_cast<const T*>(stages + (size_t)st * ATTP_STAGE_BYTES);
     const int r0 = i * RCP, rows = min(RCP, L - r0);
+    if constexpr (KA != ATTP_REG_KA)
+      attp_group_stage_scores<T, kExact, KA, CW>(Ps, i, RCP, r0, rows, A, lane, warp, ncap, act, qs, ws, e, L4, scale);
+    else
     for (int l0 = warp * 4; l0 < rows; l0 += ATTP_CWARPS * 4) {
-      float4 p[ATTP_KA][4];
+      float4 p[ATTP_REG_KA][4];
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
+      for (int k = 0; k < ATTP_REG_KA; ++k) {
         const int a = lane * 4 + 128 * k;
 #pragma unroll
         for (int u = 0; u < 4; ++u)
@@ -450,7 +528,7 @@ attention_step_fwd_group_kernel(const T* __restrict__ ann, const T* __restrict__
         if (!(act & (1u << g))) continue;
         float s4[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-        for (int k = 0; k < ATTP_KA; ++k) {
+        for (int k = 0; k < ATTP_REG_KA; ++k) {
           const int a = lane * 4 + 128 * k;
           if (a < A) {
             const float4 q4 = *reinterpret_cast<const float4*>(qs + g * A + a);
@@ -623,7 +701,7 @@ __device__ __forceinline__ uint32_t sat_pack_bf16x2(float lo, float hi) {
   return *reinterpret_cast<const uint32_t*>(&v);
 }
 
-template <bool kExact, int CW>
+template <bool kExact, int CW, int KA = ATTP_REG_KA>
 __global__ void __launch_bounds__(CW * 32 + 32, 2)
 attention_step_fwd_group_tc_kernel(const __grid_constant__ CUtensorMap tm_ann, const bf16* __restrict__ P,
                                    const float* __restrict__ wf, const float* __restrict__ hp, int64_t ldhp,
@@ -715,12 +793,14 @@ attention_step_fwd_group_tc_kernel(const __grid_constant__ CUtensorMap tm_ann, c
   for (int a = tid; a < A; a += ATTP_CONSUMERS) ws[a] = wf[a];
   sat_named_bar(1, ATTP_CONSUMERS);
 
-  float wreg[ATTP_KA][4];
+  float wreg[ATTP_REG_KA][4];
+  if constexpr (KA == ATTP_REG_KA) {
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
-    const int a = lane * 4 + 128 * k;
+    for (int k = 0; k < ATTP_REG_KA; ++k) {
+      const int a = lane * 4 + 128 * k;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+      for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+    }
   }
   int it = 0;
   for (int i = 0; i < nP; ++i, ++it) {
@@ -728,10 +808,13 @@ attention_step_fwd_group_tc_kernel(const __grid_constant__ CUtensorMap tm_ann, c
     sat_mbar_wait(&hd->full[st], (uint32_t)(it / ATTP_NST) & 1u);
     const T* Ps = reinterpret_cast<const T*>(stages + (size_t)st * ATTP_STAGE_BYTES);
     const int r0 = i * RCP, rows = min(RCP, L - r0);
+    if constexpr (KA != ATTP_REG_KA)
+      attp_group_stage_scores<T, kExact, KA, CW>(Ps, i, RCP, r0, rows, A, lane, warp, ncap, act, qs, ws, e, L4, scale);
+    else
     for (int l0 = warp * 4; l0 < rows; l0 += ATTP_CWARPS * 4) {
-      float4 p[ATTP_KA][4];
+      float4 p[ATTP_REG_KA][4];
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
+      for (int k = 0; k < ATTP_REG_KA; ++k) {
         const int a = lane * 4 + 128 * k;
 #pragma unroll
         for (int u = 0; u < 4; ++u)
@@ -741,7 +824,7 @@ attention_step_fwd_group_tc_kernel(const __grid_constant__ CUtensorMap tm_ann, c
         if (!(act & (1u << g))) continue;
         float s4[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-        for (int k = 0; k < ATTP_KA; ++k) {
+        for (int k = 0; k < ATTP_REG_KA; ++k) {
           const int a = lane * 4 + 128 * k;
           if (a < A) {
             const float4 q4 = *reinterpret_cast<const float4*>(qs + g * A + a);
@@ -874,7 +957,7 @@ attention_step_fwd_group_tc_kernel(const __grid_constant__ CUtensorMap tm_ann, c
 //   zT[d, g] = sum_l ann[l, d] * alpha[g, l]      mma.sync.m16n8k8: M = 16 columns d, N = 8 caption rows, K = 8 locations
 // so no MMA row is wasted; warp w owns columns [w*D/8, (w+1)*D/8) (MT 16-column tiles, 4 accumulator registers each).
 // =============================================================================================
-template <bool kExact, int CW, int MT>
+template <bool kExact, int CW, int MT, int KA = ATTP_REG_KA>
 __global__ void __launch_bounds__(CW * 32 + 32, 2)
 attention_step_fwd_group_tcr_kernel(const bf16* __restrict__ ann, const bf16* __restrict__ P, const float* __restrict__ wf,
                                     const float* __restrict__ hp, int64_t ldhp, const int32_t* __restrict__ lens, int t, int ncap,
@@ -972,12 +1055,14 @@ attention_step_fwd_group_tcr_kernel(const bf16* __restrict__ ann, const bf16* __
   for (int a = tid; a < A; a += ATTP_CONSUMERS) ws[a] = wf[a];
   sat_named_bar(1, ATTP_CONSUMERS);
 
-  float wreg[ATTP_KA][4];
+  float wreg[ATTP_REG_KA][4];
+  if constexpr (KA == ATTP_REG_KA) {
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
-    const int a = lane * 4 + 128 * k;
+    for (int k = 0; k < ATTP_REG_KA; ++k) {
+      const int a = lane * 4 + 128 * k;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+      for (int i = 0; i < 4; ++i) wreg[k][i] = a < A ? ws[a + i] : 0.0f;
+    }
   }
   int it = 0;
   for (int i = 0; i < nP; ++i, ++it) {
@@ -985,10 +1070,13 @@ attention_step_fwd_group_tcr_kernel(const bf16* __restrict__ ann, const bf16* __
     sat_mbar_wait(&hd->full[st], (uint32_t)(it / nst) & 1u);
     const T* Ps = reinterpret_cast<const T*>(stages + (size_t)st * stage_bytes);
     const int r0 = i * RCP, rows = min(RCP, L - r0);
+    if constexpr (KA != ATTP_REG_KA)
+      attp_group_stage_scores<T, kExact, KA, CW>(Ps, i, RCP, r0, rows, A, lane, warp, ncap, act, qs, ws, e, L4, scale);
+    else
     for (int l0 = warp * 4; l0 < rows; l0 += ATTP_CWARPS * 4) {
-      float4 p[ATTP_KA][4];
+      float4 p[ATTP_REG_KA][4];
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
+      for (int k = 0; k < ATTP_REG_KA; ++k) {
         const int a = lane * 4 + 128 * k;
 #pragma unroll
         for (int u = 0; u < 4; ++u)
@@ -998,7 +1086,7 @@ attention_step_fwd_group_tcr_kernel(const bf16* __restrict__ ann, const bf16* __
         if (!(act & (1u << g))) continue;
         float s4[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-        for (int k = 0; k < ATTP_KA; ++k) {
+        for (int k = 0; k < ATTP_REG_KA; ++k) {
           const int a = lane * 4 + 128 * k;
           if (a < A) {
             const float4 q4 = *reinterpret_cast<const float4*>(qs + g * A + a);
@@ -1275,9 +1363,9 @@ attention_step_fwd_pair_kernel(const __grid_constant__ CUtensorMap tm_ann, const
   // ===== consumers =====
   SAT_PDL_WAIT();
   const float* hp_b = hp + (int64_t)b * ldhp;
-  float qreg[ATTP_KA][4], wreg[ATTP_KA][4];
+  float qreg[ATTP_REG_KA][4], wreg[ATTP_REG_KA][4];
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
+  for (int k = 0; k < ATTP_REG_KA; ++k) {
     const int a = lane * 4 + 128 * k;
     float4 q4 = make_float4(0.f, 0.f, 0.f, 0.f), w4 = q4;
     if (a < A) {
@@ -1300,7 +1388,7 @@ attention_step_fwd_pair_kernel(const __grid_constant__ CUtensorMap tm_ann, const
     for (int lr = warp * 4; lr < rows; lr += CW * 4) {
       float s4[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
+      for (int k = 0; k < ATTP_REG_KA; ++k) {
         const int a = lane * 4 + 128 * k;
         if (a < A) {
           float4 p[4];
@@ -1442,8 +1530,9 @@ static inline size_t attention_fwd_pipe_smem(int L, int D, int A, int vn) {
          (size_t)ATTP_NST * ATTP_STAGE_BYTES;
 }
 
-// The pipelined kernel needs: one row of P and of the annotations to fit a stage, and at most 256 16-byte
-// column vectors per annotation row (D <= 2048 bf16 / 1024 fp32); other shapes use the plain kernel.
+// The pipelined kernel needs: one row of P and of the annotations to fit a stage, at most 256 16-byte column vectors per
+// annotation row (D <= 2048 bf16 / 1024 fp32) and attention_dim <= 1024 (a multiple of 4 above 256: 16-byte shared-memory
+// loads of q and w_f); other shapes use the plain kernel.
 template <typename T>
 static inline bool attention_pipe_ok(int L, int D, int A) {
   static int mode = -2;                       // SAT_ATT_MODE=0 forces the plain single-pass kernel (A/B timing)
@@ -1453,7 +1542,8 @@ static inline bool attention_pipe_ok(int L, int D, int A) {
   }
   if (mode == 0) return false;
   (void)L;
-  return D * (int)sizeof(T) <= ATTP_STAGE_BYTES && A <= 128 * ATTP_KA && D / Vec16<T>::N <= ATTP_FWD_CW * 32;
+  return D * (int)sizeof(T) <= ATTP_STAGE_BYTES && A <= 128 * ATTP_MAXKA && (A <= 128 * ATTP_REG_KA || A % 4 == 0) &&
+         D / Vec16<T>::N <= ATTP_FWD_CW * 32;
 }
 
 // launch helper shared by the training and decode drivers
@@ -1478,7 +1568,7 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
     // launch / fill / drain costs, not by the path of one row.  Kept as an opt-in variant (SAT_ATT_PAIR=1), off by default.
     static const int pair_mode = getenv("SAT_ATT_PAIR") ? atoi(getenv("SAT_ATT_PAIR")) : 0;
     const int Dh = D / 2;
-    const bool pair_fit = ncap == 1 && D % 16 == 0 && Dh <= 256 && Dh * 2 * ATTC_BOX_ROWS <= ATTP_STAGE_BYTES && A <= 128 * ATTP_KA && A % 4 == 0 &&
+    const bool pair_fit = ncap == 1 && D % 16 == 0 && Dh <= 256 && Dh * 2 * ATTC_BOX_ROWS <= ATTP_STAGE_BYTES && A <= ATTC_MAXA && A % 4 == 0 &&
                           L >= 8 && ldhp % 4 == 0 && (reinterpret_cast<uintptr_t>(hp) & 15) == 0;
     if (pair_fit && (pair_mode == 1 || (pair_mode != 0 && rows <= 3 * 148))) {
       static thread_local CUtensorMap tmp;
@@ -1508,13 +1598,17 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
                          (size_t)ncap * (((D / Vec16<T>::N) >= ATTP_FWD_CW * 32 ? 1 : (ATTP_FWD_CW * 32) / (D / Vec16<T>::N)) * (size_t)D) *
                                  sizeof(float) <= (size_t)ATTP_NST * ATTP_STAGE_BYTES;
   const bool group = group_fit && (group_mode == 1 || (group_mode != 0 && (size_t)L * D * sizeof(T) >= SAT_ATT_GROUP_MIN_BYTES));
+  // kernel instantiation for the attention_dim: KA column slices of 128 per lane
+  const int ka = attp_ka(A);
+  auto by_ka = [ka](auto k2, auto k4, auto k8) { return ka == 2 ? k2 : (ka == 4 ? k4 : k8); };
   if constexpr (std::is_same<T, bf16>::value && !kExact) {
     static const int group_tc_mode = getenv("SAT_ATT_GROUP_TC") ? atoi(getenv("SAT_ATT_GROUP_TC")) : 1;
     if (group && group_tc_mode != 0 && D % ATTG_BOX_COLS == 0 && ld_z % 2 == 0 && ldhp % 2 == 0 && A % 2 == 0) {
+      // a variant whose shared memory (it grows with A) exceeds the per-block limit falls back to the next one
       static const int tcr_mode = getenv("SAT_ATT_GROUP_TCR") ? atoi(getenv("SAT_ATT_GROUP_TCR")) : 1;
       // measured: row-streamed 89 vs box 100 us at D=2048 (C5), but 49 vs 43 us at D=512 (1 KB rows: too many small copies)
-      if ((tcr_mode == 2 || (tcr_mode == 1 && D >= 1024)) && (D == 512 || D == 1024 || D == 2048)) {
-        const AttTcrGeom gm = attention_fwd_group_tcr_geom(L, D, A);
+      const AttTcrGeom gm = attention_fwd_group_tcr_geom(L, D, A);
+      if ((tcr_mode == 2 || (tcr_mode == 1 && D >= 1024)) && (D == 512 || D == 1024 || D == 2048) && gm.smem <= ATTP_SMEM_MAX) {
         auto launch_r = [&](auto kern) -> int {
           SAT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gm.smem));
           SAT_CUDA(sat_launch_pdl(kern, dim3(rows / ncap), dim3(ATTP_FWD_CW * 32 + 32), gm.smem, st, ann, P, wf, hp, ldhp, lens, t, ncap, L, D,
@@ -1522,11 +1616,16 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
           SAT_COUNT_LAUNCH();
           return 0;
         };
-        if (D == 512) return launch_r(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 4>);
-        if (D == 1024) return launch_r(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 8>);
-        return launch_r(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 16>);
+        if (D == 512)
+          return launch_r(by_ka(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 4, 2>, attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 4, 4>,
+                                attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 4, 8>));
+        if (D == 1024)
+          return launch_r(by_ka(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 8, 2>, attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 8, 4>,
+                                attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 8, 8>));
+        return launch_r(by_ka(attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 16, 2>, attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 16, 4>,
+                              attention_step_fwd_group_tcr_kernel<kExact, ATTP_FWD_CW, 16, 8>));
       }
-      if (L <= 16 * ATTG_MAXKS) {
+      if (L <= 16 * ATTG_MAXKS && attention_fwd_group_tc_smem(L, A) <= ATTP_SMEM_MAX) {
       // annotations as a 2-D tensor [n_img * L, D]; the map is rebuilt only when the buffer or shape changes
       static thread_local CUtensorMap tm;
       static thread_local const void* tm_ptr = nullptr;
@@ -1539,7 +1638,8 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
         SAT_TRY(tc::make_map(&tm, ann, n_rows, D, D, ATTG_BOX_ROWS));
         tm_ptr = ann; tm_rows = n_rows; tm_d = D; tm_dev = dev_now;
       }
-      auto kern = attention_step_fwd_group_tc_kernel<kExact, ATTP_FWD_CW>;
+      auto kern = by_ka(attention_step_fwd_group_tc_kernel<kExact, ATTP_FWD_CW, 2>, attention_step_fwd_group_tc_kernel<kExact, ATTP_FWD_CW, 4>,
+                        attention_step_fwd_group_tc_kernel<kExact, ATTP_FWD_CW, 8>);
       const size_t smem = attention_fwd_group_tc_smem(L, A);
       SAT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       SAT_CUDA(sat_launch_pdl(kern, dim3(rows / ncap), dim3(ATTP_FWD_CW * 32 + 32), smem, st, tm, P, wf, hp, ldhp, lens, t, ncap, L, D, A,
@@ -1549,7 +1649,8 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
       }
     }
   }
-  if (group) {
+  const size_t gsmem = ncap <= 3 ? attention_fwd_group_smem<3>(L, A) : (ncap <= 5 ? attention_fwd_group_smem<5>(L, A) : attention_fwd_group_smem<8>(L, A));
+  if (group && gsmem <= ATTP_SMEM_MAX) {
     auto launch_g = [&](auto kern, size_t smem) -> int {
       SAT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       SAT_CUDA(sat_launch_pdl(kern, dim3(rows / ncap), dim3(ATTP_FWD_CW * 32 + 32), smem, st, ann, P, wf, hp, ldhp, lens, t, ncap, L, D, A,
@@ -1557,12 +1658,18 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
       SAT_COUNT_LAUNCH();
       return 0;
     };
-    if (ncap <= 3) return launch_g(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 3>, attention_fwd_group_smem<3>(L, A));
-    if (ncap <= 5) return launch_g(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 5>, attention_fwd_group_smem<5>(L, A));
-    return launch_g(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 8>, attention_fwd_group_smem<8>(L, A));
+    if (ncap <= 3)
+      return launch_g(by_ka(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 3, 2>, attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 3, 4>,
+                            attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 3, 8>), gsmem);
+    if (ncap <= 5)
+      return launch_g(by_ka(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 5, 2>, attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 5, 4>,
+                            attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 5, 8>), gsmem);
+    return launch_g(by_ka(attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 8, 2>, attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 8, 4>,
+                          attention_step_fwd_group_kernel<T, kExact, ATTP_FWD_CW, 8, 8>), gsmem);
   }
   const size_t smem = attention_fwd_pipe_smem(L, D, A, Vec16<T>::N);
-  auto kern = attention_step_fwd_pipe_kernel<T, kExact, ATTP_FWD_CW>;
+  auto kern = by_ka(attention_step_fwd_pipe_kernel<T, kExact, ATTP_FWD_CW, 2>, attention_step_fwd_pipe_kernel<T, kExact, ATTP_FWD_CW, 4>,
+                    attention_step_fwd_pipe_kernel<T, kExact, ATTP_FWD_CW, 8>);
   // set on every launch (sub-microsecond): a per-translation-unit cache of "largest value set so far" is wrong here, because the
   // kernel is one function for the whole library while this launcher is compiled into several translation units -- another
   // unit's launcher may have lowered the attribute in between (seen as "invalid argument" in a long mixed train / decode run)
@@ -1583,11 +1690,14 @@ static int launch_attention_fwd(const T* ann, const T* P, const float* wf, const
 //     D: u = tanh(P + q) recomputed from the P stages; dP += dpu (fp32 read-modify-write, 4 rows in flight per warp),
 //        dq = sum_l dpu, dwf partial
 //   Same math and summation structure per row as attention_step_bwd_kernel (kept as the fallback).
+//   KA > 2 (A > 256): in phase D warp w owns the 128-column slice w % KA for the rows w / KA, w / KA + CW / KA, .. of every
+//   stage (KA <= CW), so its dq / dwf accumulators stay 8 registers and every warp works on every stage, however few P rows
+//   a stage holds.  q and w_f of the slice are read from shared memory once.
 // =============================================================================================
 constexpr int ATTB_MAXSEG = 4;   // column segments per annotation row (segmented phase B)
 constexpr int ATTB_VPL = 4;      // 16-byte annotation vectors per lane kept in registers (D <= 1024 bf16 / 512 fp32)
 
-template <typename T, bool kExact, int CW>
+template <typename T, bool kExact, int CW, int KA = ATTP_REG_KA>
 __global__ void __launch_bounds__(CW * 32 + 32, 2)      // two CTAs per SM: all B=256 captions resident in one wave
 attention_step_bwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ P, const float* __restrict__ wf,
                                const float* __restrict__ q_t, const float* __restrict__ alpha, int64_t ld_alpha,
@@ -1824,10 +1934,72 @@ attention_step_bwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
   }
   sat_named_bar(1, ATTP_CONSUMERS);
 
-  // phase D: through tanh into P, q, wf (lane owns attention columns lane*4 + 128k)
-  float qreg[ATTP_KA][4], wreg[ATTP_KA][4], dq[ATTP_KA][4], dw[ATTP_KA][4];
+  if constexpr (KA != ATTP_REG_KA) {
+    static_assert(KA <= CW && CW % KA == 0, "one column slice per warp");
+    // phase D, KA > 2: warp w owns columns 128 * (w % KA) + lane * 4 .. +3 for the 4-row groups rsub, rsub + RS, .. of a stage
+    constexpr int RS = CW / KA;
+    const int ks = warp % KA, rsub = warp / KA;
+    const int a = lane * 4 + 128 * ks;
+    const bool own = a < A;
+    float4 q4 = make_float4(0.f, 0.f, 0.f, 0.f), w4 = q4;
+    if (own) {
+      q4 = *reinterpret_cast<const float4*>(qs + a);
+      w4 = *reinterpret_cast<const float4*>(ws + a);
+    }
+    const float qv[4] = {q4.x, q4.y, q4.z, q4.w}, wv[4] = {w4.x, w4.y, w4.z, w4.w};
+    float dq[4] = {0.f, 0.f, 0.f, 0.f}, dw[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int j = 0; j < nP; ++j, ++it) {
+      const int st = it % ATTP_NST;
+      sat_mbar_wait(&hd->full[st], (uint32_t)(it / ATTP_NST) & 1u);
+      const T* Ps = reinterpret_cast<const T*>(stages + (size_t)st * ATTP_STAGE_BYTES);
+      const int r0 = j * RCP, rows = min(RCP, L - r0);
+      if (own) {
+        for (int l0 = rsub * 4; l0 < rows; l0 += RS * 4) {
+          float4 p[4];
+          float de[4];
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
+          for (int u = 0; u < 4; ++u) {
+            const bool ok = (l0 + u) < rows;
+            p[u] = ok ? ld4(Ps + (size_t)(l0 + u) * A + a) : make_float4(0.f, 0.f, 0.f, 0.f);
+            de[u] = ok ? dal[r0 + l0 + u] : 0.0f;
+          }
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const float pv[4] = {p[u].x, p[u].y, p[u].z, p[u].w};
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              const float uu = sat_tanh<kExact>(pv[i] + qv[i]);
+              dq[i] = fmaf(de[u] * wv[i], 1.0f - uu * uu, dq[i]);
+              dw[i] = fmaf(de[u], uu, dw[i]);
+            }
+          }
+        }
+      }
+      __syncwarp();
+      if (lane == 0) sat_mbar_arrive(&hd->empty[st]);
+    }
+    sat_named_bar(1, ATTP_CONSUMERS);     // every warp is done reading the ring before red[] overwrites it
+    if (own) {
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        red[rsub * 2 * A + a + i] = dq[i];
+        red[rsub * 2 * A + A + a + i] = dw[i];
+      }
+    }
+    sat_named_bar(1, ATTP_CONSUMERS);
+    for (int a2 = tid; a2 < A; a2 += ATTP_CONSUMERS) {
+      float sq = 0.0f, sw = 0.0f;
+#pragma unroll
+      for (int r = 0; r < RS; ++r) { sq += red[r * 2 * A + a2]; sw += red[r * 2 * A + A + a2]; }
+      dy_b[a2] = from_f<T>(sq);
+      dwf_t[(int64_t)b * A + a2] = sw;
+    }
+    return;
+  }
+  // phase D: through tanh into P, q, wf (lane owns attention columns lane*4 + 128k)
+  float qreg[ATTP_REG_KA][4], wreg[ATTP_REG_KA][4], dq[ATTP_REG_KA][4], dw[ATTP_REG_KA][4];
+#pragma unroll
+  for (int k = 0; k < ATTP_REG_KA; ++k) {
     const int a = lane * 4 + 128 * k;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -1846,7 +2018,7 @@ attention_step_bwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
     const int r0 = j * RCP, rows = min(RCP, L - r0);
     for (int l0 = warp * 4; l0 < rows; l0 += ATTP_CWARPS * 4) {      // 4 rows in flight per warp
 #pragma unroll
-      for (int k = 0; k < ATTP_KA; ++k) {
+      for (int k = 0; k < ATTP_REG_KA; ++k) {
         const int a = lane * 4 + 128 * k;
         if (a < A) {
           float4 p[4];
@@ -1875,7 +2047,7 @@ attention_step_bwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
   }
   sat_named_bar(1, ATTP_CONSUMERS);     // every warp is done reading the ring before red[] overwrites it
 #pragma unroll
-  for (int k = 0; k < ATTP_KA; ++k) {
+  for (int k = 0; k < ATTP_REG_KA; ++k) {
     const int a = lane * 4 + 128 * k;
     if (a < A) {
 #pragma unroll
@@ -1897,20 +2069,23 @@ attention_step_bwd_pipe_kernel(const T* __restrict__ ann, const T* __restrict__ 
 
 // dP[b,l,a] = sum_t de[t,b,l] * w_f[a] * (1 - tanh^2(P[img,l,a] + q[t,b,a])), t = lens[b]-1 .. 0: the grad wrt the
 // per-image projection P, rebuilt once after the time loop (model.py:100-104 under autograd).  One CTA per (row tile,
-// caption): q[:,b,:] and de[:,b,tile] are staged in smem, every warp walks 4 rows at a time, a lane owns 4 columns.
+// caption, column chunk): q[:,b,chunk] and de[:,b,tile] are staged in smem, every warp walks 4 rows at a time, a lane owns
+// 4 columns.  The column chunk (AC columns, a multiple of 128, or all of A) bounds the staged q at Tmax * AC floats.
 constexpr int DPD_ROWS = 32;
-template <typename T, bool kExact>
-__global__ void __launch_bounds__(256, 4)
+template <typename T, bool kExact, bool kCols>
+__global__ void __launch_bounds__(256, kCols ? 1 : 4)     // kCols: the staged q fills most of the shared memory of an SM
 dP_deferred_kernel(const T* __restrict__ P, const float* __restrict__ wf, const float* __restrict__ Q,
                    const float* __restrict__ de, const int32_t* __restrict__ lens, int ncap, int B, int L, int A, int Tmax,
-                   float* __restrict__ dP, T* __restrict__ dP16) {
+                   float* __restrict__ dP, T* __restrict__ dP16, int ac_arg) {
   extern __shared__ __align__(16) float dpd_smem[];
   const int b = blockIdx.y, r0 = blockIdx.x * DPD_ROWS, rows = min(DPD_ROWS, L - r0);
+  const int AC = kCols ? ac_arg : A;                                    // !kCols: one chunk, all of A
+  const int a0 = kCols ? (int)blockIdx.z * AC : 0, nac = kCols ? min(AC, A - a0) : A;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int Tb = min(lens[b], Tmax);    // shared memory is sized for Tmax steps
-  float* qs = dpd_smem;                       // [Tb][A]
-  float* des = qs + (size_t)Tb * A;           // [Tb][DPD_ROWS]
-  for (int i = tid; i < Tb * A; i += 256) qs[i] = Q[((int64_t)(i / A) * B + b) * A + (i % A)];
+  float* qs = dpd_smem;                       // [Tb][AC]
+  float* des = qs + (size_t)Tb * AC;          // [Tb][DPD_ROWS]
+  for (int i = tid; i < Tb * nac; i += 256) qs[(i / nac) * AC + (i % nac)] = Q[((int64_t)(i / nac) * B + b) * A + a0 + (i % nac)];
   for (int i = tid; i < Tb * DPD_ROWS; i += 256) {
     const int t = i / DPD_ROWS, l = i % DPD_ROWS;
     des[i] = l < rows ? de[((int64_t)t * B + b) * L + r0 + l] : 0.0f;
@@ -1919,7 +2094,7 @@ dP_deferred_kernel(const T* __restrict__ P, const float* __restrict__ wf, const 
   const T* Pb = P + ((int64_t)(b / ncap) * L + r0) * A;
   const int l0 = warp * 4;
   if (l0 >= rows) return;
-  for (int a = lane * 4; a < A; a += 128) {
+  for (int a = a0 + lane * 4; a < a0 + nac; a += 128) {
     const float4 w4 = *reinterpret_cast<const float4*>(wf + a);
     const float wv[4] = {w4.x, w4.y, w4.z, w4.w};
     float pv[4][4], acc[4][4];
@@ -1931,7 +2106,7 @@ dP_deferred_kernel(const T* __restrict__ P, const float* __restrict__ wf, const 
       for (int i = 0; i < 4; ++i) acc[u][i] = 0.0f;
     }
     for (int t = Tb - 1; t >= 0; --t) {
-      const float4 q4 = *reinterpret_cast<const float4*>(qs + (size_t)t * A + a);
+      const float4 q4 = *reinterpret_cast<const float4*>(qs + (size_t)t * AC + (a - a0));
       const float qv[4] = {q4.x, q4.y, q4.z, q4.w};
       const float4 d4 = *reinterpret_cast<const float4*>(des + (size_t)t * DPD_ROWS + l0);
       const float dv[4] = {d4.x, d4.y, d4.z, d4.w};
@@ -1962,6 +2137,16 @@ static inline size_t attention_bwd_pipe_smem(int L, int D, int A) {
          (size_t)ATTP_NST * ATTP_STAGE_BYTES;
 }
 
+// dP_deferred_kernel: columns per CTA so that q of Tmax steps fits the shared memory of a block (all of A when it fits, as
+// many 128-column slices as fit otherwise); 0 where not even one slice fits (the step-by-step backward kernel runs instead)
+static inline int dP_deferred_cols(int T, int A) {
+  auto bytes = [T](int ac) { return sizeof(float) * (size_t)T * (ac + DPD_ROWS); };
+  if (bytes(A) <= ATTP_SMEM_MAX) return A;
+  int ac = 128;
+  while (ac + 128 < A && bytes(ac + 128) <= ATTP_SMEM_MAX) ac += 128;
+  return bytes(ac) <= ATTP_SMEM_MAX ? ac : 0;
+}
+
 template <typename T>
 static inline bool attention_bwd_pipe_ok(int D, int A) {
   static int mode = -2;                       // SAT_ATTB_MODE=0 forces the plain kernel (A/B timing)
@@ -1970,5 +2155,5 @@ static inline bool attention_bwd_pipe_ok(int D, int A) {
     mode = e ? atoi(e) : -1;
   }
   if (mode == 0) return false;
-  return D * (int)sizeof(T) <= ATTP_STAGE_BYTES && A <= 128 * ATTP_KA;
+  return D * (int)sizeof(T) <= ATTP_STAGE_BYTES && A <= 128 * ATTP_MAXKA;
 }

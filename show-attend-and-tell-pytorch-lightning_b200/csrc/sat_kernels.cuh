@@ -574,9 +574,11 @@ __global__ void lstm_bwd_step_kernel(const TS* __restrict__ gates, const float* 
 //   dP[b,l,a] += dpu ;  dq_a = sum_l dpu_la ;  dwf_a = scale * sum_l de_l u_la
 // Algorithmic traffic per active row: L*(A+D)*sizeof(T) read + 2*L*A*4 (dP read-modify-write).
 // =============================================================================================
-constexpr int ATTB_MAXKA = 4;   // attention_dim <= 512
+// A lane keeps dq / dwf of the attention columns lane*4 + 128k, k < KA, in registers: the instantiation for KA serves
+// attention_dim <= 128 * KA (KA = 4: A <= 512, KA = 8: A <= 1024, the training limit).
+constexpr int ATTB_MAXKA = 8;   // attention_dim <= 1024
 
-template <typename T, bool kExact>
+template <typename T, bool kExact, int KA = 4>
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_step_bwd_kernel(const T* __restrict__ ann, const T* __restrict__ P, const float* __restrict__ wf,
                           const float* __restrict__ q_t, const float* __restrict__ alpha, int64_t ld_alpha,
@@ -655,15 +657,15 @@ attention_step_bwd_kernel(const T* __restrict__ ann, const T* __restrict__ P, co
   // phase D: through tanh into P, q, wf
   const T* Pb = P + (int64_t)img * L * A;
   float* dPb = dP + (int64_t)b * L * A;
-  float dq[ATTB_MAXKA][4], dw[ATTB_MAXKA][4];
+  float dq[KA][4], dw[KA][4];
 #pragma unroll
-  for (int k = 0; k < ATTB_MAXKA; ++k)
+  for (int k = 0; k < KA; ++k)
 #pragma unroll
     for (int i = 0; i < 4; ++i) { dq[k][i] = 0.0f; dw[k][i] = 0.0f; }
   for (int l = warp; l < L; l += NW) {
     const float de = dal[l] * scale;
 #pragma unroll
-    for (int k = 0; k < ATTB_MAXKA; ++k) {
+    for (int k = 0; k < KA; ++k) {
       const int a = lane * 4 + k * 128;
       if (a < A) {
         const float4 p = ld4(Pb + (int64_t)l * A + a);
@@ -685,7 +687,7 @@ attention_step_bwd_kernel(const T* __restrict__ ann, const T* __restrict__ P, co
     }
   }
 #pragma unroll
-  for (int k = 0; k < ATTB_MAXKA; ++k) {
+  for (int k = 0; k < KA; ++k) {
     const int a = lane * 4 + k * 128;
     if (a < A) {
 #pragma unroll

@@ -59,13 +59,19 @@ int train_backward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& 
   const float scale = (float)(1.0 / sqrt((double)L));
   // pipelined attention backward: saves de_t per step and dP is rebuilt once after the loop (dP_deferred_kernel);
   // the plain kernel accumulates dP step by step and needs it zeroed
-  const bool att_pipe = attention_bwd_pipe_ok<TS>(D, A) && b.de != nullptr && A % 4 == 0;
+  const int dpd_cols = dP_deferred_cols(T, A);
+  const bool att_pipe = attention_bwd_pipe_ok<TS>(D, A) && b.de != nullptr && A % 4 == 0 && dpd_cols > 0;
   if (!att_pipe) {
     SAT_CUDA(cudaMemsetAsync(b.dP, 0, sizeof(float) * (size_t)B * L * A, st));
     if (dann_tc) SAT_CUDA(cudaMemsetAsync(b.dP16, 0, sizeof(TS) * (size_t)B * L * A, st));
   }
   const size_t att_smem = att_pipe ? attention_bwd_pipe_smem(L, D, A) : attention_bwd_smem(L, D, A);
-  auto att_k = att_pipe ? attention_step_bwd_pipe_kernel<TS, kExact, ATTP_BWD_CW> : attention_step_bwd_kernel<TS, kExact>;
+  // instantiation by attention_dim: 128-column slices per lane (pipelined: 2 / 4 / 8; step-by-step kernel: 4 / 8)
+  const int ka = attp_ka(A);
+  auto att_k = att_pipe ? (ka == 2 ? attention_step_bwd_pipe_kernel<TS, kExact, ATTP_BWD_CW, 2>
+                                   : (ka == 4 ? attention_step_bwd_pipe_kernel<TS, kExact, ATTP_BWD_CW, 4>
+                                              : attention_step_bwd_pipe_kernel<TS, kExact, ATTP_BWD_CW, 8>))
+                        : (A <= 512 ? attention_step_bwd_kernel<TS, kExact, 4> : attention_step_bwd_kernel<TS, kExact, 8>);
   const int att_threads = att_pipe ? ATTP_BWD_CW * 32 + 32 : ATT_THREADS;
   if (att_smem > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(att_k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
 
@@ -125,11 +131,11 @@ int train_backward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& 
   }
 
   if (att_pipe) {
-    const size_t sm = sizeof(float) * (size_t)T * (A + DPD_ROWS);
-    auto kp = dP_deferred_kernel<TS, kExact>;
+    const size_t sm = sizeof(float) * (size_t)T * (dpd_cols + DPD_ROWS);
+    auto kp = dpd_cols == A ? dP_deferred_kernel<TS, kExact, false> : dP_deferred_kernel<TS, kExact, true>;
     if (sm > 48 * 1024) SAT_CUDA(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    kp<<<dim3((L + DPD_ROWS - 1) / DPD_ROWS, B), 256, sm, st>>>((const TS*)b.P, w.wf, b.Q, b.de, b.lens, d.ncap, B, L, A, T, b.dP,
-                                                              dann_tc ? (TS*)b.dP16 : (TS*)nullptr);
+    kp<<<dim3((L + DPD_ROWS - 1) / DPD_ROWS, B, (A + dpd_cols - 1) / dpd_cols), 256, sm, st>>>(
+        (const TS*)b.P, w.wf, b.Q, b.de, b.lens, d.ncap, B, L, A, T, b.dP, dann_tc ? (TS*)b.dP16 : (TS*)nullptr, dpd_cols);
     SAT_COUNT_LAUNCH();
     SAT_LAUNCH_OK();
   }
@@ -195,7 +201,7 @@ int train_backward_impl(const SatDims& d, const SatWeights& w, SatTrainBuffers& 
 
 extern "C" int sat_train_backward(const SatDims* d, const SatWeights* w, SatTrainBuffers* b, void* stream) {
   SAT_REQUIRE(d && w && b, "sat_train_backward: NULL struct");
-  SAT_REQUIRE(d->A <= 128 * ATTB_MAXKA, "sat_train_backward: attention_dim %d > %d", d->A, 128 * ATTB_MAXKA);
+  SAT_REQUIRE(d->A <= 128 * ATTB_MAXKA, "sat_train_backward: attention_dim %d exceeds the training limit of %d", d->A, 128 * ATTB_MAXKA);
   SAT_REQUIRE(b->dlogits && b->gscale && b->dpre && b->dHZ && b->DY && b->dgz && b->dh && b->dc && b->dZ && b->dP &&
                   b->dwf_part && b->dXe && b->d_init_out && b->df1 && b->dmean && b->d_ann,
               "sat_train_backward: NULL backward buffer");
