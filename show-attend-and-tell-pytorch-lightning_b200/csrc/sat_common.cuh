@@ -225,6 +225,10 @@ template <bool kExact> __device__ __forceinline__ float sat_sigmoid(float x) {
   return __fdividef(1.0f, 1.0f + __expf(-x));
 }
 
+// A word id as the kernels use it: ids outside [0, V0) (nn.Embedding would raise) are fed and scored as <PAD> (id 0);
+// tok_init_kernel flags such a caption in out[6].  The one rule for the fed words and both cross-entropy paths' targets.
+__device__ __forceinline__ int sat_word_or_pad(int w, int V0) { return (unsigned)w < (unsigned)V0 ? w : 0; }
+
 // ---- dropout: stateless counter-based masks ------------------------------------------------------
 // keep(seed, stream, idx) is a pure function, so the backward pass regenerates the forward masks instead of storing them.
 // streams: 1 = InitLSTM mean (model.py:78), 2 = embedding_dropout (model.py:526), 3 = DeepOutput dropout (model.py:130)

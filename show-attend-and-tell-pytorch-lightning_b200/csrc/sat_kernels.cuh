@@ -287,12 +287,9 @@ static __global__ void tok_init_kernel(const int32_t* __restrict__ caps, int32_t
   const int m = blockIdx.x * blockDim.x + threadIdx.x;
   if (m >= T_ * B) return;
   const int t = m / B, b = m - t * B;
-  int w = caps[(int64_t)b * caplen + t];
-  if ((unsigned)w >= (unsigned)V0) {      // nn.Embedding would raise; here the word is fed as <PAD> and the step is flagged (out[6])
-    w = 0;
-    *err_flag = 1.0f;
-  }
-  tok[m] = w;
+  const int w = caps[(int64_t)b * caplen + t];
+  if ((unsigned)w >= (unsigned)V0) *err_flag = 1.0f;     // nn.Embedding would raise; here the word is fed as <PAD>, flagged (out[6])
+  tok[m] = sat_word_or_pad(w, V0);
 }
 
 // the dataset hands out int64 word ids / lengths (torch.LongTensor, util.py:43-44); the kernels index with int32
@@ -389,8 +386,7 @@ ce_rows_kernel(TL* __restrict__ logits, TD* __restrict__ dlogits, const int32_t*
     if (tid == 0) { row_loss[m] = 0.0f; row_argmax[m] = -1; }
     return;
   }
-  int y = caps[(int64_t)b * caplen + t + 1];
-  if ((unsigned)y >= (unsigned)V0) y = 0;      // out-of-range target ids are flagged by tok_init_kernel (out[6])
+  const int y = sat_word_or_pad(caps[(int64_t)b * caplen + t + 1], V0);
   float mx = -INFINITY, sx = 0.0f;
   int arg = 0x7fffffff;
   for (int v = tid * 4; v < V; v += 256 * 4) {      // 4 logits per access (rows are 16 B (bf16) / 32 B (fp32) aligned)

@@ -102,7 +102,7 @@ struct EpiVocab {
     } else {
       const int mg = a.row0 + m, t = mg / a.B, b = mg - t * a.B;
       active = active && t < a.lens[b];
-      if (active) y = a.caps[(int64_t)b * a.caplen + t + 1];
+      if (active) y = sat_word_or_pad(a.caps[(int64_t)b * a.caplen + t + 1], a.V0);
     }
     const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16) + (uint32_t)cbase;
     const bool tile_full = n0 + BN <= a.V0;                        // no padded / out-of-range column in this tile (CTA-uniform)
@@ -484,7 +484,7 @@ ss_feedback_kernel(const float4* __restrict__ stats, int NT, const int32_t* __re
   if (b >= B || t - 1 >= lens[b]) return;
   float mx;
   const int arg = tiles_argmax(stats + (int64_t)b * NT, NT, lane, mx);
-  if (lane == 0) tok_t[b] = (unsigned)arg < (unsigned)V0 ? arg : 0;
+  if (lane == 0) tok_t[b] = sat_word_or_pad(arg, V0);
 }
 
 // Greedy decode: candidate (score, word) of every live row from the tile statistics -- the k = 1 output of
